@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the per-cube compress+decompress hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = hyper-mode encode + decode of every 64^3 cube of the synthetic vox10 cloud (BASELINE
@@ -135,12 +135,13 @@ class ClockSampler(threading.Thread):
 def device_step(codec, st):
     """All GPU kernels of encode + decode on device-resident inputs, issued exactly as the product issues them
     (transform.encode_on_device / _decompress_hyper_gpu_coder: conv transforms on the main stream, the GPU range coder on the
-    coder stream).  Not in here: the host range coding of the one hyper string z and the PCIe copies -- those are in ``e2e``."""
+    coder stream).  Not in here: the host range coding of the one hyper string z and the PCIe copies -- those are in ``e2e``.
+    -> the step's results as device tensors, still being computed (read them after a device synchronise)."""
     from pcgcv1_b200 import transform
     eb, cem = st["eb"], st["cem"]
     codec.deferred_checks(True)
     try:
-        _, _, z_hats, _, _, _, _ = transform.encode_on_device(codec, eb, cem, st["cubes"], want_likelihoods=True)
+        _, mm, z_hats, _, packed, offsets, _ = transform.encode_on_device(codec, eb, cem, st["cubes"], want_likelihoods=True)
         # decode side: headers (min/max) and the strings come from the stream, z_hat from the (host) hyper decoder
         z_all = torch_cat(z_hats)
         xs = transform._decompress_hyper_gpu_coder(codec, cem, None, st["mins"], st["maxs"], [1, 16, 16, 16, 16],
@@ -149,7 +150,46 @@ def device_step(codec, st):
     finally:
         codec.deferred_checks(False)
     mask, _, cnt = codec.topk(xs.raw, st["ks"])                 # same stream as the synthesis: stream order is enough
-    return mask, cnt
+    return {"y_strings_packed": packed, "y_string_offsets": offsets, "y_minmax": mm, "z_hat": z_all, "occupancy_logits": xs.raw,
+            "occupancy": mask, "voxel_counts": cnt}
+
+
+# --dump-outputs: name -> (dtype written, most elements written); 62 MB in all at most.  The strings of the vox10 cloud (8.0 MB)
+# fit whole, so any change of the latents shows; indices, offsets and counts are float64 so that they stay exact.
+DUMP_ARRAYS = {"y_strings": (np.float32, 1 << 23), "y_string_offsets": (np.float64, 1 << 16), "y_minmax": (np.float64, 1 << 17),
+               "z_hat": (np.float32, 1 << 20), "occupancy_logits": (np.float32, 1 << 21), "occupied_voxels": (np.float64, 1 << 21),
+               "voxel_counts": (np.float64, 1 << 16)}
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def step_outputs(out):
+    """device_step's tensors (complete: after a device synchronise) -> the arrays a caller of the path receives: the strings
+    (bytes, concatenated; string b = y_strings[off[b]:off[b+1]]), their offsets, the per-cube symbol ranges, the quantised
+    hyper-latents, the decoded occupancy logits, the flat indices of the occupied voxels of the [B,64,64,64] masks and the
+    voxels set per cube."""
+    import torch
+    end = int(out["y_string_offsets"][-1])
+    return {"y_strings": out["y_strings_packed"][:end], "y_string_offsets": out["y_string_offsets"], "y_minmax": out["y_minmax"],
+            "z_hat": out["z_hat"], "occupancy_logits": out["occupancy_logits"],
+            "occupied_voxels": torch.nonzero(out["occupancy"].reshape(-1)).reshape(-1), "voxel_counts": out["voxel_counts"]}
+
+
+def dump_outputs(arrays, directory):
+    """Writes every array of DUMP_ARRAYS as ``directory/<name>.npy``, flattened.  An array longer than its cap is replaced by the
+    elements at a fixed seeded sample of positions (kept in order; the same positions for the same length), so that two builds
+    run with the same arguments can be compared element for element."""
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    total = 0
+    for name, (dtype, cap) in DUMP_ARRAYS.items():
+        t = arrays[name].reshape(-1)
+        if t.numel() > cap:
+            pos = np.sort(np.random.default_rng(0).choice(t.numel(), cap, replace=False))
+            t = t[torch.from_numpy(pos).to(t.device)]
+        a = t.cpu().numpy().astype(dtype)
+        np.save(os.path.join(directory, name + ".npy"), a)
+        total += a.nbytes
+    assert total <= DUMP_LIMIT_BYTES, total
 
 
 def device_step_transforms(codec, st):
@@ -266,11 +306,20 @@ def run_gpu(args):
     codec.profile(True)
     codec.profile_report()
     l0 = codec.launch_count()
-    dev_ms, _ = timed(lambda: device_step(codec, st), args.steps, 0)
+    last = {}
+
+    def value_step():
+        last["out"] = device_step(codec, st)
+    dev_ms, _ = timed(value_step, args.steps, 0)
     launches = codec.launch_count() - l0
     prof = codec.profile_report()
     codec.profile(False)
     clocks = sampler.finish()
+    out = last.pop("out")
+    if args.dump_outputs and rank == 0:
+        codec.synchronize()                                     # raises if a kernel of the timed steps flagged an error
+        dump_outputs(step_outputs(out), args.dump_outputs)
+    del out
     # the same kernels without the range coder (the r01 definition of value, for comparison across rounds)
     nocoder_steps = max(3, args.steps // 2)
     nocoder_ms, _ = timed(lambda: device_step_transforms(codec, st), nocoder_steps, 1)
@@ -740,7 +789,14 @@ def main():
                          "3 vox12 cloud sharded over --gpus (strong scaling), 4 analysis+synthesis batch sweep, 5 training step (batch 8)")
     ap.add_argument("--distortion", default="bce", choices=["bce", "focal"],
                     help="config 5: occupancy loss of the training step (bce = what train_hyper.py calls; focal = loss.py:83-93)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="config 1: write what the last timed step computed (strings, symbol ranges, hyper-latents, occupancy "
+                         "logits and masks) as DIR/<name>.npy, float32 / float64, a seeded sample of the larger ones, <= 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config != 1 or args.impl != "ours"):
+        ap.error("--dump-outputs applies to --config 1 with --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:
