@@ -319,6 +319,18 @@ int pcgc_voxelize(pcgc_ctx* ctx, const int16_t* local_dev, const int64_t* offset
 int pcgc_extract_points(pcgc_ctx* ctx, const uint8_t* mask_dev, int B, int S, int32_t* counts_dev, int16_t* points_dev,
                         int64_t cap, int64_t* total_dev);
 
+/* ---- D1 / D2 geometry metrics (myutils/pc_error_wrapper.py geometry_metrics; MPEG pc_error's definitions) ------------------
+ * a_dev float64 [n_a,3], b_dev float64 [n_b,3], normals_a_dev float64 [n_a,3] (unit normals of A) or NULL for p2point only; all
+ * DEVICE pointers.  For direction 1 every a against its nearest b, for direction 2 every b against its nearest a; e = query - neighbour:
+ *   p2point |e|^2,  p2plane (e . n)^2 with n = normal of a (direction 1) or of the nearest a (direction 2).
+ * out_dev double[8] = [direction 1, 2][p2point, p2plane][sum, max]; the p2plane entries are 0 when normals_a_dev is NULL.
+ * Exact search (uniform grid over each set, ring-by-ring, no cap).  TIE RULE: among equidistant neighbours the lowest index of the
+ * searched array wins.  Per-point arithmetic as NumPy's ((x0 + x1) + x2, no contraction); sums in a fixed order (deterministic;
+ * exact for integer coordinates).  Empty sets or more than 2^27 points: PCGC_ERR_BAD_ARG.  Enqueued on the ctx stream, does not
+ * synchronise (except when the per-ctx workspace grows). */
+int pcgc_geometry_sums(pcgc_ctx* ctx, const double* a_dev, int64_t n_a, const double* b_dev, int64_t n_b, const double* normals_a_dev,
+                       double* out_dev);
+
 #ifdef __cplusplus
 }
 #endif

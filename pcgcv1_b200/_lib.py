@@ -91,6 +91,7 @@ SIGNATURES = {
     "pcgc_partition_points": (_i, [_vp, _i64, _i, _i, _vp, _i64, _vp, _vp, _vp, _vp, _vp]),
     "pcgc_voxelize": (_i, [_vp, _vp, _vp, _i, _i, _vp]),
     "pcgc_extract_points": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i64, _vp]),
+    "pcgc_geometry_sums": (_i, [_vp, _vp, _i64, _vp, _i64, _vp, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None

@@ -129,4 +129,14 @@ cudaError_t launch_voxelize(const int16_t* local, const int64_t* offsets, int B,
 cudaError_t launch_extract_points(const uint8_t* mask, int B, int S, int64_t* chunk_ws, int32_t* counts, int16_t* points, int64_t cap,
                                   int64_t* total, cudaStream_t s, int64_t* launches);
 
+// metrics.cu: nearest-neighbour geometry sums with a per-ctx workspace (grown on demand, freed with the ctx)
+struct GeoWorkspace;
+// the grids of A and B (sized for na / nb points; the workspace is reused by the next launch_geometry_queries) ...
+cudaError_t launch_geometry_grids(GeoWorkspace** ws, const double* a, int64_t na, const double* b, int64_t nb, cudaStream_t s,
+                                  int64_t* launches);
+// ... then both directions' nearest-neighbour queries and the sums into out double[8]
+cudaError_t launch_geometry_queries(GeoWorkspace* ws, const double* a, const double* b, const double* normals_a, double* out, cudaStream_t s,
+                                    int64_t* launches);
+void free_geometry_workspace(GeoWorkspace* ws);
+
 }  // namespace pcgc

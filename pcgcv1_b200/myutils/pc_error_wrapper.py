@@ -81,6 +81,22 @@ def _load_xyz_normals(filename):
     return xyz, normals
 
 
+def _figures(stats, peak):
+    """``stats[kind][side] = (mse, h)`` for kind in p2point[, p2plane] and side "1" / "2" -> the dict of HEADERS keys."""
+    psnr = lambda v: float("inf") if v == 0 else 10.0 * np.log10(3.0 * peak * peak / v)
+    out = {}
+    for kind in stats:
+        for side in ("1", "2"):
+            mse, h = stats[kind][side]
+            out["h.       %s(%s)" % (side, kind)], out["h.,PSNR  %s(%s)" % (side, kind)] = h, psnr(h)
+            out["mse%s      (%s)" % (side, kind)], out["mse%s,PSNR (%s)" % (side, kind)] = mse, psnr(mse)
+        hf = max(out["h.       1(%s)" % kind], out["h.       2(%s)" % kind])
+        mf = max(out["mse1      (%s)" % kind], out["mse2      (%s)" % kind])
+        out["h.        (%s)" % kind], out["h.,PSNR   (%s)" % kind] = hf, psnr(hf)
+        out["mseF      (%s)" % kind], out["mseF,PSNR (%s)" % kind] = mf, psnr(mf)
+    return out
+
+
 def geometry_metrics(a, b, normals_a=None, peak=1023.0):
     """The 24 figures of ``pc_error -a A -b B -n N --hausdorff=1 --resolution=peak`` from their definitions (module docstring).
     ``a`` [n,3], ``b`` [m,3]; ``normals_a`` [n,3] or None (then the p2plane keys are absent, as when the tool runs without -n)."""
@@ -96,18 +112,28 @@ def geometry_metrics(a, b, normals_a=None, peak=1023.0):
         na = np.asarray(normals_a, np.float64)
         d["1"]["p2plane"] = ((e1 * na).sum(1)) ** 2
         d["2"]["p2plane"] = ((e2 * na[ib]).sum(1)) ** 2
-    psnr = lambda v: float("inf") if v == 0 else 10.0 * np.log10(3.0 * peak * peak / v)
-    out = {}
-    for kind in d["1"]:
-        for side in ("1", "2"):
-            h, mse = float(d[side][kind].max()), float(d[side][kind].mean())
-            out["h.       %s(%s)" % (side, kind)], out["h.,PSNR  %s(%s)" % (side, kind)] = h, psnr(h)
-            out["mse%s      (%s)" % (side, kind)], out["mse%s,PSNR (%s)" % (side, kind)] = mse, psnr(mse)
-        hf = max(out["h.       1(%s)" % kind], out["h.       2(%s)" % kind])
-        mf = max(out["mse1      (%s)" % kind], out["mse2      (%s)" % kind])
-        out["h.        (%s)" % kind], out["h.,PSNR   (%s)" % kind] = hf, psnr(hf)
-        out["mseF      (%s)" % kind], out["mseF,PSNR (%s)" % kind] = mf, psnr(mf)
-    return out
+    return _figures({kind: {side: (float(d[side][kind].mean()), float(d[side][kind].max())) for side in ("1", "2")} for kind in d["1"]},
+                    peak)
+
+
+def geometry_metrics_device(a, b, normals_a=None, peak=1023.0, codec=None):
+    """``geometry_metrics`` on the GPU (``Codec.geometry_sums``: exact grid search, lowest index of the searched set on ties):
+    the same keys and the same mean / max / PSNR expressions.  ``a``, ``b``, ``normals_a``: [n,3] torch tensors (moved to the
+    codec's device as float64 if they are not there) or arrays.  For integer coordinates the p2point figures equal
+    ``geometry_metrics``' bit for bit; the p2plane figures can differ where the nearest neighbour is not unique (the k-d tree's
+    tie order is unspecified)."""
+    import torch
+    from .. import runtime
+    c = codec or runtime.get_codec("voxception", "")
+    a, b = c.to_device(a, torch.float64), c.to_device(b, torch.float64)
+    n = None if normals_a is None else c.to_device(normals_a, torch.float64)
+    if len(a) == 0 or len(b) == 0:
+        raise ValueError("geometry_metrics: empty point cloud")
+    s = runtime.to_host(c.geometry_sums(a, b, n), "geometry_sums").reshape(2, 2, 2).astype(np.float64)
+    count = {"1": len(a), "2": len(b)}
+    kinds = ("p2point",) if n is None else ("p2point", "p2plane")
+    return _figures({kind: {side: (float(s[int(side) - 1, k, 0]) / count[side], float(s[int(side) - 1, k, 1])) for side in ("1", "2")}
+                     for k, kind in enumerate(kinds)}, peak)
 
 
 def pc_error(infile1, infile2, normal1, res, show=False):

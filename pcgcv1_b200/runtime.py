@@ -596,6 +596,12 @@ class Codec:
         """uint8 mask [B,S,S,S(,1)] on the device -> (points int16 [total,3] NumPy, counts int32 [B] NumPy): the non-zero
         voxels of every cube in np.where order (voxels2points, inout_points.py:134-143).  ``cap`` = an upper bound of the
         total when the caller knows one (saves a second pass)."""
+        pts, counts = self.extract_points_device(mask, cap)
+        return to_host(pts, "extract_points").copy(), to_host(counts, "extract_counts").copy()
+
+    def extract_points_device(self, mask: torch.Tensor, cap: Optional[int] = None):
+        """extract_points with the results left on the device: (points int16 [total,3], counts int32 [B]) torch tensors.
+        Synchronises once to read the total."""
         B, S = mask.shape[0], mask.shape[1]
         counts = torch.empty(max(B, 1), dtype=torch.int32, device=self.dev)
         total = torch.empty(1, dtype=torch.int64, device=self.dev)
@@ -608,7 +614,26 @@ class Codec:
             if t <= n:
                 break
             cap = t
-        return to_host(pts[:t], "extract_points").copy(), to_host(counts[:B], "extract_counts").copy()
+        return pts[:t], counts[:B]
+
+    def geometry_sums(self, a: torch.Tensor, b: torch.Tensor, normals_a: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """D1 / D2 sums of two point sets on the device (pcgc_geometry_sums): a, b float64 [n,3] (normals_a float64 [n_a,3] or
+        None) on this codec's device -> float64 [2,2,2] device tensor [direction 1 (a -> b), 2 (b -> a)][p2point, p2plane][sum,
+        max] (p2plane zero without normals).  Asynchronous on the current stream."""
+        for name, t in (("a", a), ("b", b), ("normals_a", normals_a)):
+            if t is None:
+                continue
+            if t.dtype != torch.float64 or t.dim() != 2 or t.shape[1] != 3 or t.device != self.dev or not t.is_contiguous():
+                raise ValueError("%s must be a contiguous float64 [n,3] tensor on %s" % (name, self.dev))
+        if len(a) == 0 or len(b) == 0:
+            raise ValueError("geometry_sums: empty point cloud")
+        if normals_a is not None and len(normals_a) != len(a):
+            raise ValueError("normals_a must have one row per point of a")
+        out = torch.empty((2, 2, 2), dtype=torch.float64, device=self.dev)
+        self._stream()
+        self._check(self.lib.pcgc_geometry_sums(self.ctx, a.data_ptr(), len(a), b.data_ptr(), len(b),
+                                                normals_a.data_ptr() if normals_a is not None else None, out.data_ptr()))
+        return out
 
     def count_voxels(self, cubes: torch.Tensor) -> np.ndarray:
         """number of non-zero voxels per cube (np.sum(cubes, axis=(1,2,3,4)), process.py:44)."""

@@ -24,6 +24,8 @@ _OPTIONS = [
     ("--gpu", int, 1, "kept for compatibility; must be 1"),
 ]
 
+CUBE_SIZE_MESSAGE = "the transforms are built for 64^3 cubes (the reference's default and its checkpoints)"
+
 
 def parse_args(argv=None):
     ap = argparse.ArgumentParser(prog="pcgcv1_b200.test", formatter_class=argparse.ArgumentDefaultsHelpFormatter)
@@ -89,7 +91,7 @@ def main(argv=None):
     if args.gpu != 1:
         raise SystemExit("pcgcv1_b200 has no CPU path (--gpu 0): the codec is the CUDA library")
     if args.cube_size != 64:
-        raise SystemExit("the transforms are built for 64^3 cubes (the reference's default and its checkpoints)")
+        raise SystemExit(CUBE_SIZE_MESSAGE)
     session = _Session(args)
     getattr(session, args.command)()
 
