@@ -331,6 +331,23 @@ int pcgc_extract_points(pcgc_ctx* ctx, const uint8_t* mask_dev, int B, int S, in
 int pcgc_geometry_sums(pcgc_ctx* ctx, const double* a_dev, int64_t n_a, const double* b_dev, int64_t n_b, const double* normals_a_dev,
                        double* out_dev);
 
+/* ---- k-nearest-neighbour PCA normals of one point set (the normals file D2 reads) ---------------------------------------------
+ * pts_dev float64 [n,3], normals_dev float64 [n,3] (out), knn_idx_dev int32 [n,k] (out, optional: NULL = not written); all DEVICE
+ * pointers.  1 <= n <= 2^27, 1 <= k <= 64 (k > n: all n points); otherwise PCGC_ERR_BAD_ARG.
+ *   NEIGHBOURHOOD of point i: the m = min(k, n) points of the set with the smallest (d2, index), compared lexicographically, with
+ *     e = p_i - p_j and d2 = (e0*e0 + e1*e1) + e2*e2 (as pcgc_geometry_sums).  The point itself is included (d2 = 0); equidistant
+ *     points are taken in ascending index (the LOWEST index wins at the k-th distance).  knn_idx_dev row i lists them in that
+ *     order; slots m .. k-1 hold -1.  Exact search over one uniform grid (pcgc_geometry_sums' grid and ring-by-ring search, no cap).
+ *   COVARIANCE, in (d2, index) order, on u_j = p_j - p_i (relative to the point, which leaves C unchanged mathematically and keeps
+ *     it exactly 0 when all neighbours coincide): mu = (sum u_j) / m, then C = sum (u_j - mu)(u_j - mu)^T / m; two passes, running
+ *     sums in that fixed order, every multiply and add rounded on its own (no FMA).
+ *   NORMAL: the unit eigenvector of the smallest eigenvalue of C by cyclic Jacobi (at most 32 sweeps; lowest axis on an exact
+ *     eigenvalue tie), scaled to unit length; sign: its component of largest magnitude is positive (lowest axis on an exact tie).
+ *     C == 0 (one point, or all neighbours at the same coordinates) gives (0, 0, 1).
+ * Deterministic (two calls give the same bits).  Enqueued on the ctx stream, does not synchronise (except when the per-ctx
+ * workspace, shared with pcgc_geometry_sums, grows). */
+int pcgc_estimate_normals(pcgc_ctx* ctx, const double* pts_dev, int64_t n, int k, double* normals_dev, int32_t* knn_idx_dev);
+
 #ifdef __cplusplus
 }
 #endif

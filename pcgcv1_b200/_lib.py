@@ -92,6 +92,7 @@ SIGNATURES = {
     "pcgc_voxelize": (_i, [_vp, _vp, _vp, _i, _i, _vp]),
     "pcgc_extract_points": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i64, _vp]),
     "pcgc_geometry_sums": (_i, [_vp, _vp, _i64, _vp, _i64, _vp, _vp]),
+    "pcgc_estimate_normals": (_i, [_vp, _vp, _i64, _i, _vp, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None

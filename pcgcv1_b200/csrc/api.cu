@@ -1478,6 +1478,20 @@ int pcgc_geometry_sums(pcgc_ctx* ctx, const double* a_dev, int64_t n_a, const do
   return PCGC_OK;
 }
 
+int pcgc_estimate_normals(pcgc_ctx* ctx, const double* pts_dev, int64_t n, int k, double* normals_dev, int32_t* knn_idx_dev) {
+  if (!ctx || !pts_dev || !normals_dev || n <= 0 || n > ((int64_t)1 << 27) || k < 1 || k > 64)
+    return fail(ctx, PCGC_ERR_BAD_ARG, "pcgc_estimate_normals: bad argument (1 .. 2^27 points, 1 <= k <= 64)");
+  DeviceGuard g(ctx->device);
+  prof_begin(ctx, "normals_grid", 0, 24.0 * (double)n + 32.0 * (double)n);
+  CK(launch_normals_grid(&ctx->geo_ws, pts_dev, n, ctx->stream, &ctx->launches));
+  prof_end(ctx);
+  const int kk = (int)std::min<int64_t>(k, n);
+  prof_begin(ctx, "normals_query", 0, (double)n * (32.0 + 2.0 * 24.0 * kk + 24.0 + (knn_idx_dev ? 4.0 * k : 0.0)));
+  CK(launch_normals_query(ctx->geo_ws, pts_dev, n, k, normals_dev, knn_idx_dev, ctx->stream, &ctx->launches));
+  prof_end(ctx);
+  return PCGC_OK;
+}
+
 int pcgc_widen_symbol_ranges(pcgc_ctx* ctx, int32_t* minmax_dev, int n_pairs) {
   if (!ctx || !minmax_dev || n_pairs < 0) return fail(ctx, PCGC_ERR_BAD_ARG, "pcgc_widen_symbol_ranges: bad argument");
   DeviceGuard g(ctx->device);

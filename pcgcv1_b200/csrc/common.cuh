@@ -138,5 +138,10 @@ cudaError_t launch_geometry_grids(GeoWorkspace** ws, const double* a, int64_t na
 cudaError_t launch_geometry_queries(GeoWorkspace* ws, const double* a, const double* b, const double* normals_a, double* out, cudaStream_t s,
                                     int64_t* launches);
 void free_geometry_workspace(GeoWorkspace* ws);
+// k-nearest-neighbour PCA normals of one set, in the same workspace: its grid ...
+cudaError_t launch_normals_grid(GeoWorkspace** ws, const double* p, int64_t n, cudaStream_t s, int64_t* launches);
+// ... then per point the k nearest (d2, index), the covariance and its smallest eigenvector (knn may be null)
+cudaError_t launch_normals_query(GeoWorkspace* ws, const double* p, int64_t n, int k, double* normals, int32_t* knn, cudaStream_t s,
+                                 int64_t* launches);
 
 }  // namespace pcgc

@@ -1,6 +1,7 @@
 // D1 / D2 geometry sums (myutils/pc_error_wrapper.py geometry_metrics) on the device: exact nearest neighbours through a uniform
 // grid, per-point p2point / p2plane values in NumPy's arithmetic, and a fixed-order reduction.  Contract in include/pcgc_b200.h
-// (pcgc_geometry_sums).
+// (pcgc_geometry_sums).  The same grid and search, widened from one to k nearest neighbours, give the PCA normals of
+// pcgc_estimate_normals (knn_normals_kernel).
 //
 // Grid over a searched set S (n points):
 //   - cell size h = the smallest (to 1e-9 relative) for which the dense table has at most kCellsPerPoint * n cells, found by bisection
@@ -8,7 +9,8 @@
 //   - points sorted by linear cell id with a stable radix sort, so the points of a cell are contiguous and in ascending index order;
 //     a row of cells along x is one contiguous range of the sorted points;
 //   - a coarse occupancy level (kCoarse^3 fine cells per coarse cell) bounds the cost of far queries (Hausdorff outliers): after
-//     kFineRings fine rings the search continues ring by ring over the coarse cells and skips the empty ones.
+//     kFineRings fine rings the search continues ring by ring over the coarse cells and skips the empty ones (and the fine rows
+//     already scanned, so that no point is visited twice).
 // A query q is first clamped to the bounding box (q'); for every p of S, |q - p|^2 >= |q - q'|^2 + |q' - p|^2, and the points of the
 // cells outside a ring of radius r around the cell of q' are at least `lb` from q', lb = distance from q' to that ring's outer faces
 // on the sides where the grid continues (less a slack of 1e-12 of the grid's coordinate range for the rounding of the cell index).
@@ -181,6 +183,59 @@ __device__ __forceinline__ bool done_after(const GridParams& g, double lb, doubl
   return (dq2 + lb * lb) * (1.0 - 1e-12) > best;
 }
 
+// The exact search around the query qc (clamped to the bounding box, |q - qc|^2 = dq2) in cell c: every fine ring r = 0..kFineRings,
+// then every coarse ring over the occupied coarse cells, skipping the fine rows already scanned, so that every point is visited at most
+// once.  scan(j0, j1) visits the sorted points [j0, j1); the walk ends when done_after holds for bound() (the d2 an unvisited point
+// must beat) or no cell is left.
+template <class Scan, class Bound>
+__device__ __forceinline__ void ring_search(const GridParams& g, const int32_t* __restrict__ starts, const int32_t* __restrict__ coarse,
+                                            const double* qc, const int* c, double dq2, Scan&& scan, Bound&& bound) {
+  const int Gx = g.G[0], Gy = g.G[1];
+  bool done = false;
+  for (int r = 0; r <= kFineRings && !done; ++r) {
+    for (int z = max(c[2] - r, 0); z <= min(c[2] + r, g.G[2] - 1); ++z)
+      for (int y = max(c[1] - r, 0); y <= min(c[1] + r, Gy - 1); ++y) {
+        const int64_t base = ((int64_t)z * Gy + y) * Gx;
+        if (abs(z - c[2]) == r || abs(y - c[1]) == r) {
+          const int x0 = max(c[0] - r, 0), x1 = min(c[0] + r, Gx - 1);
+          scan(starts[base + x0], starts[base + x1 + 1]);
+        } else {
+          if (c[0] - r >= 0) scan(starts[base + c[0] - r], starts[base + c[0] - r + 1]);
+          if (c[0] + r < Gx) scan(starts[base + c[0] + r], starts[base + c[0] + r + 1]);
+        }
+      }
+    done = done_after(g, outside_distance(g, qc, c, r, g.h, g.G), dq2, bound());
+  }
+  if (done) return;
+  const int R = kFineRings;
+  const int cc[3] = {c[0] / kCoarse, c[1] / kCoarse, c[2] / kCoarse};
+  const int Cx = g.Gc[0], Cy = g.Gc[1], Cz = g.Gc[2];
+  for (int r = 0; !done; ++r) {
+    for (int z = max(cc[2] - r, 0); z <= min(cc[2] + r, Cz - 1); ++z)
+      for (int y = max(cc[1] - r, 0); y <= min(cc[1] + r, Cy - 1); ++y) {
+        const bool full = abs(z - cc[2]) == r || abs(y - cc[1]) == r;
+        const int xa = max(cc[0] - r, 0), xb = min(cc[0] + r, Cx - 1);
+        for (int x = xa; x <= xb; ++x) {
+          if (!full && x != cc[0] - r && x != cc[0] + r) continue;     // inner rows: only the two end cells are on the ring
+          if (coarse[((int64_t)z * Cy + y) * Cx + x] == 0) continue;
+          const int fx0 = x * kCoarse, fx1 = min(fx0 + kCoarse, Gx) - 1;
+          for (int fz = z * kCoarse; fz < min(z * kCoarse + kCoarse, g.G[2]); ++fz)
+            for (int fy = y * kCoarse; fy < min(y * kCoarse + kCoarse, Gy); ++fy) {
+              const int64_t base = ((int64_t)fz * Gy + fy) * Gx;
+              if (abs(fz - c[2]) <= R && abs(fy - c[1]) <= R) {            // a row through the fine box: only the cells outside it
+                const int l1 = min(fx1, c[0] - R - 1), r0 = max(fx0, c[0] + R + 1);
+                if (fx0 <= l1) scan(starts[base + fx0], starts[base + l1 + 1]);
+                if (r0 <= fx1) scan(starts[base + r0], starts[base + fx1 + 1]);
+              } else {
+                scan(starts[base + fx0], starts[base + fx1 + 1]);
+              }
+            }
+        }
+      }
+    done = done_after(g, outside_distance(g, qc, cc, r, g.hc, g.Gc), dq2, bound());
+  }
+}
+
 // One thread per query.  Queries come in the cell order of their own set (neighbouring threads search neighbouring cells).
 // dir 1: normal of the query (normals[qi]); dir 2: normal of the neighbour found (normals[bi]).
 __global__ void __launch_bounds__(kThreads, 3) query_kernel(const SortedPoint* __restrict__ queries, int64_t nq, const GridParams* __restrict__ gp,
@@ -202,45 +257,9 @@ __global__ void __launch_bounds__(kThreads, 3) query_kernel(const SortedPoint* _
     dq2 = dq2 + d * d;
     c[k] = cell_of(qc[k], g.lo[k], g.inv_h, g.G[k]);
   }
-  const int Gx = g.G[0], Gy = g.G[1];
   Best b;
-  bool done = false;
-  for (int r = 0; r <= kFineRings && !done; ++r) {
-    for (int z = max(c[2] - r, 0); z <= min(c[2] + r, g.G[2] - 1); ++z)
-      for (int y = max(c[1] - r, 0); y <= min(c[1] + r, Gy - 1); ++y) {
-        const int64_t base = ((int64_t)z * Gy + y) * Gx;
-        if (abs(z - c[2]) == r || abs(y - c[1]) == r) {
-          const int x0 = max(c[0] - r, 0), x1 = min(c[0] + r, Gx - 1);
-          scan_range(pts, starts[base + x0], starts[base + x1 + 1], q[0], q[1], q[2], b);
-        } else {
-          if (c[0] - r >= 0) scan_range(pts, starts[base + c[0] - r], starts[base + c[0] - r + 1], q[0], q[1], q[2], b);
-          if (c[0] + r < Gx) scan_range(pts, starts[base + c[0] + r], starts[base + c[0] + r + 1], q[0], q[1], q[2], b);
-        }
-      }
-    done = done_after(g, outside_distance(g, qc, c, r, g.h, g.G), dq2, b.d2);
-  }
-  if (!done) {
-    const int cc[3] = {c[0] / kCoarse, c[1] / kCoarse, c[2] / kCoarse};
-    const int Cx = g.Gc[0], Cy = g.Gc[1], Cz = g.Gc[2];
-    for (int r = 0; !done; ++r) {
-      for (int z = max(cc[2] - r, 0); z <= min(cc[2] + r, Cz - 1); ++z)
-        for (int y = max(cc[1] - r, 0); y <= min(cc[1] + r, Cy - 1); ++y) {
-          const bool full = abs(z - cc[2]) == r || abs(y - cc[1]) == r;
-          const int xa = max(cc[0] - r, 0), xb = min(cc[0] + r, Cx - 1);
-          for (int x = xa; x <= xb; ++x) {
-            if (!full && x != cc[0] - r && x != cc[0] + r) continue;     // inner rows: only the two end cells are on the ring
-            if (coarse[((int64_t)z * Cy + y) * Cx + x] == 0) continue;
-            const int fx0 = x * kCoarse, fx1 = min(fx0 + kCoarse, Gx) - 1;
-            for (int fz = z * kCoarse; fz < min(z * kCoarse + kCoarse, g.G[2]); ++fz)
-              for (int fy = y * kCoarse; fy < min(y * kCoarse + kCoarse, Gy); ++fy) {
-                const int64_t base = ((int64_t)fz * Gy + fy) * Gx;
-                scan_range(pts, starts[base + fx0], starts[base + fx1 + 1], q[0], q[1], q[2], b);
-              }
-          }
-        }
-      done = done_after(g, outside_distance(g, qc, cc, r, g.hc, g.Gc), dq2, b.d2);
-    }
-  }
+  ring_search(g, starts, coarse, qc, c, dq2, [&](int j0, int j1) { scan_range(pts, j0, j1, q[0], q[1], q[2], b); },
+              [&]() { return b.d2; });
   const double* p = searched + 3 * (int64_t)b.idx;
   const double e0 = q[0] - p[0], e1 = q[1] - p[1], e2 = q[2] - p[2];
   pp[qi] = (e0 * e0 + e1 * e1) + e2 * e2;
@@ -249,6 +268,134 @@ __global__ void __launch_bounds__(kThreads, 3) query_kernel(const SortedPoint* _
     const double en = (e0 * nn[0] + e1 * nn[1]) + e2 * nn[2];
     pl[qi] = en * en;
   }
+}
+
+// ---- k nearest neighbours and PCA normals (pcgc_estimate_normals) -------------------------------------------------------------------
+// One thread per query, queries in the cell order of the set.  The k best (d2, index) pairs are kept sorted in a per-thread array of
+// CAP slots (CAP = 16, 32 or 64 >= k): local memory, since it is indexed dynamically.
+template <int CAP>
+struct KBest {
+  double d2[CAP];
+  int idx[CAP];
+  int count = 0;       // slots held (<= kk)
+  int kk;              // min(k, n)
+  __device__ __forceinline__ double kth() const { return count >= kk ? d2[kk - 1] : DBL_MAX; }
+};
+
+template <int CAP>
+__device__ __forceinline__ void knn_scan(const SortedPoint* __restrict__ pts, int j0, int j1, const double* q, KBest<CAP>& b) {
+  for (int j = j0; j < j1; ++j) {
+    const SortedPoint p = pts[j];
+    const double e0 = q[0] - p.x, e1 = q[1] - p.y, e2 = q[2] - p.z;
+    const double d2 = (e0 * e0 + e1 * e1) + e2 * e2;
+    const int idx = (int)p.idx;
+    if (b.count == b.kk) {
+      const double w = b.d2[b.kk - 1];
+      if (!(d2 < w || (d2 == w && idx < b.idx[b.kk - 1]))) continue;
+    }
+    int pos = b.count < b.kk ? b.count : b.kk - 1;
+    while (pos > 0 && (d2 < b.d2[pos - 1] || (d2 == b.d2[pos - 1] && idx < b.idx[pos - 1]))) {
+      b.d2[pos] = b.d2[pos - 1]; b.idx[pos] = b.idx[pos - 1]; --pos;
+    }
+    b.d2[pos] = d2; b.idx[pos] = idx;
+    if (b.count < b.kk) ++b.count;
+  }
+}
+
+// Cyclic Jacobi on the symmetric 3x3 matrix A (overwritten), at most kJacobiSweeps sweeps; returns the unit eigenvector of
+// the smallest eigenvalue (lowest axis on an exact tie of eigenvalues) with the sign rule of the header.
+constexpr int kJacobiSweeps = 32;
+
+__device__ void smallest_eigenvector(double A[3][3], double* out) {
+  double V[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}};
+  const int P[3] = {0, 0, 1}, Q[3] = {1, 2, 2};
+  for (int sweep = 0; sweep < kJacobiSweeps; ++sweep) {
+    if (A[0][1] == 0.0 && A[0][2] == 0.0 && A[1][2] == 0.0) break;
+    for (int r = 0; r < 3; ++r) {
+      const int p = P[r], q = Q[r], o = 3 - p - q;
+      const double apq = A[p][q];
+      if (apq == 0.0) continue;
+      const double g = 100.0 * fabs(apq);
+      if (sweep > 3 && fabs(A[p][p]) + g == fabs(A[p][p]) && fabs(A[q][q]) + g == fabs(A[q][q])) {
+        A[p][q] = A[q][p] = 0.0;                     // below the rounding of both diagonal entries
+        continue;
+      }
+      const double h = A[q][q] - A[p][p];
+      double t;
+      if (fabs(h) + g == fabs(h)) {
+        t = apq / h;
+      } else {
+        const double theta = 0.5 * h / apq;
+        t = 1.0 / (fabs(theta) + sqrt(1.0 + theta * theta));
+        if (theta < 0.0) t = -t;
+      }
+      const double c = 1.0 / sqrt(1.0 + t * t), sn = t * c, tau = sn / (1.0 + c);
+      A[p][p] = A[p][p] - t * apq;
+      A[q][q] = A[q][q] + t * apq;
+      A[p][q] = A[q][p] = 0.0;
+      const double gp = A[o][p], gq = A[o][q];
+      A[o][p] = A[p][o] = gp - sn * (gq + gp * tau);
+      A[o][q] = A[q][o] = gq + sn * (gp - gq * tau);
+      for (int i = 0; i < 3; ++i) {
+        const double vp = V[i][p], vq = V[i][q];
+        V[i][p] = vp - sn * (vq + vp * tau);
+        V[i][q] = vq + sn * (vp - vq * tau);
+      }
+    }
+  }
+  int m = 0;
+  for (int i = 1; i < 3; ++i)
+    if (A[i][i] < A[m][m]) m = i;
+  double v[3] = {V[0][m], V[1][m], V[2][m]};
+  const double inv = 1.0 / sqrt((v[0] * v[0] + v[1] * v[1]) + v[2] * v[2]);
+  int a = 0;
+  for (int i = 0; i < 3; ++i) {
+    v[i] = v[i] * inv;
+    if (fabs(v[i]) > fabs(v[a])) a = i;
+  }
+  const double sg = v[a] < 0.0 ? -1.0 : 1.0;
+  for (int i = 0; i < 3; ++i) out[i] = v[i] * sg + 0.0;     // + 0.0: no negative zeros
+}
+
+template <int CAP>
+__global__ void __launch_bounds__(kThreads) knn_normals_kernel(const SortedPoint* __restrict__ pts, int64_t n, int k,
+                                                               const GridParams* __restrict__ gp, const int32_t* __restrict__ starts,
+                                                               const int32_t* __restrict__ coarse, const double* __restrict__ src,
+                                                               double* __restrict__ normals, int32_t* __restrict__ knn) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  const GridParams g = *gp;
+  const SortedPoint qp = pts[t];
+  const double q[3] = {qp.x, qp.y, qp.z};      // a point of the set: inside the bounding box, so no clamping
+  const int qi = (int)qp.idx;
+  int c[3];
+  for (int d = 0; d < 3; ++d) c[d] = cell_of(q[d], g.lo[d], g.inv_h, g.G[d]);
+  KBest<CAP> b;
+  b.kk = (int)min((int64_t)k, n);
+  ring_search(g, starts, coarse, q, c, 0.0, [&](int j0, int j1) { knn_scan(pts, j0, j1, q, b); }, [&]() { return b.kth(); });
+  const int m = b.count;
+  if (knn)
+    for (int j = 0; j < k; ++j) knn[(int64_t)qi * k + j] = j < m ? b.idx[j] : -1;
+  // Covariance about the centroid, in coordinates relative to the query (u = p - q): two passes in (d2, index) order.
+  double mu[3] = {0.0, 0.0, 0.0};
+  for (int j = 0; j < m; ++j) {
+    const double* p = src + 3 * (int64_t)b.idx[j];
+    for (int d = 0; d < 3; ++d) mu[d] = mu[d] + (p[d] - q[d]);
+  }
+  for (int d = 0; d < 3; ++d) mu[d] = mu[d] / (double)m;
+  double C[3][3] = {{0.0, 0.0, 0.0}, {0.0, 0.0, 0.0}, {0.0, 0.0, 0.0}};
+  for (int j = 0; j < m; ++j) {
+    const double* p = src + 3 * (int64_t)b.idx[j];
+    const double e[3] = {(p[0] - q[0]) - mu[0], (p[1] - q[1]) - mu[1], (p[2] - q[2]) - mu[2]};
+    for (int u = 0; u < 3; ++u)
+      for (int v = u; v < 3; ++v) C[u][v] = C[u][v] + e[u] * e[v];
+  }
+  for (int u = 0; u < 3; ++u)
+    for (int v = u; v < 3; ++v) C[v][u] = C[u][v] = C[u][v] / (double)m;
+  double nrm[3] = {0.0, 0.0, 1.0};
+  if (C[0][0] != 0.0 || C[0][1] != 0.0 || C[0][2] != 0.0 || C[1][1] != 0.0 || C[1][2] != 0.0 || C[2][2] != 0.0)
+    smallest_eigenvector(C, nrm);
+  for (int d = 0; d < 3; ++d) normals[3 * (int64_t)qi + d] = nrm[d];
 }
 
 // Stage 1: block b sums / maxes the contiguous chunk b of the n values of each of `nv` arrays (fixed tree); stage 2 folds the
@@ -325,22 +472,33 @@ struct Plan {
   size_t sort_bytes = 0, scan_bytes = 0;
 };
 
+void carve_grid(Carver& c, Grid& g, int64_t n) {
+  const size_t cells = (size_t)kCellsPerPoint * n + 8;
+  g.params = c.take<GridParams>(1);
+  g.partial = c.take<double>(kRedBlocks * 6);
+  for (int k = 0; k < 2; ++k) { g.keys[k] = c.take<uint32_t>(n); g.vals[k] = c.take<int32_t>(n); }
+  g.counts = c.take<int32_t>(cells);
+  g.starts = c.take<int32_t>(cells + 1);
+  g.coarse = c.take<int32_t>(cells);
+  g.pts = c.take<SortedPoint>(n);
+}
+
 size_t carve(char* base, Plan& p) {
   Carver c{base};
   for (int s = 0; s < 2; ++s) {
-    const size_t cells = (size_t)kCellsPerPoint * p.n[s] + 8;
-    Grid& g = p.g[s];
-    g.params = c.take<GridParams>(1);
-    g.partial = c.take<double>(kRedBlocks * 6);
-    for (int k = 0; k < 2; ++k) { g.keys[k] = c.take<uint32_t>(p.n[s]); g.vals[k] = c.take<int32_t>(p.n[s]); }
-    g.counts = c.take<int32_t>(cells);
-    g.starts = c.take<int32_t>(cells + 1);
-    g.coarse = c.take<int32_t>(cells);
-    g.pts = c.take<SortedPoint>(p.n[s]);
+    carve_grid(c, p.g[s], p.n[s]);
     p.pp[s] = c.take<double>(p.n[s]);
     p.pl[s] = c.take<double>(p.n[s]);
   }
   p.red = c.take<double>(2 * kRedBlocks * 2);
+  p.tmp = c.take<char>(std::max(p.sort_bytes, p.scan_bytes));
+  return c.off + 256;
+}
+
+// The normals use one grid (p.g[0] over p.n[0] points) and the sort / scan scratch.
+size_t carve_normals(char* base, Plan& p) {
+  Carver c{base};
+  carve_grid(c, p.g[0], p.n[0]);
   p.tmp = c.take<char>(std::max(p.sort_bytes, p.scan_bytes));
   return c.off + 256;
 }
@@ -386,19 +544,20 @@ void free_geometry_workspace(GeoWorkspace* ws) {
   delete ws;
 }
 
-cudaError_t launch_geometry_grids(GeoWorkspace** wsp, const double* a, int64_t na, const double* b, int64_t nb, cudaStream_t s,
-                                  int64_t* launches) {
-  Plan plan;
-  plan.n[0] = na; plan.n[1] = nb;
-  const int64_t nmax = std::max(na, nb);
+namespace {
+
+// CUB scratch sizes for grids of up to nmax points.
+cudaError_t size_scratch(Plan& plan, int64_t nmax, cudaStream_t s) {
   const size_t cells_max = (size_t)kCellsPerPoint * nmax + 8;
-  {
-    cub::DoubleBuffer<uint32_t> k(nullptr, nullptr);
-    cub::DoubleBuffer<int32_t> v(nullptr, nullptr);
-    GK(cub::DeviceRadixSort::SortPairs(nullptr, plan.sort_bytes, k, v, (int)nmax, 0, 32, s));
-    GK(cub::DeviceScan::ExclusiveSum(nullptr, plan.scan_bytes, (int32_t*)nullptr, (int32_t*)nullptr, (int)(cells_max + 1), s));
-  }
-  const size_t need = carve(nullptr, plan);
+  cub::DoubleBuffer<uint32_t> k(nullptr, nullptr);
+  cub::DoubleBuffer<int32_t> v(nullptr, nullptr);
+  GK(cub::DeviceRadixSort::SortPairs(nullptr, plan.sort_bytes, k, v, (int)nmax, 0, 32, s));
+  GK(cub::DeviceScan::ExclusiveSum(nullptr, plan.scan_bytes, (int32_t*)nullptr, (int32_t*)nullptr, (int)(cells_max + 1), s));
+  return cudaSuccess;
+}
+
+// Grows the workspace to `need` bytes (synchronises only then); *base = its 256-byte aligned start.
+cudaError_t reserve(GeoWorkspace** wsp, size_t need, cudaStream_t s, char** base) {
   if (!*wsp) *wsp = new GeoWorkspace();
   GeoWorkspace* ws = *wsp;
   if (ws->cap < need) {
@@ -407,7 +566,21 @@ cudaError_t launch_geometry_grids(GeoWorkspace** wsp, const double* a, int64_t n
     GK(cudaMalloc(&ws->mem, want));
     ws->cap = want;
   }
-  carve(reinterpret_cast<char*>(((uintptr_t)ws->mem + 255) & ~(uintptr_t)255), plan);
+  *base = reinterpret_cast<char*>(((uintptr_t)ws->mem + 255) & ~(uintptr_t)255);
+  return cudaSuccess;
+}
+
+}  // namespace
+
+cudaError_t launch_geometry_grids(GeoWorkspace** wsp, const double* a, int64_t na, const double* b, int64_t nb, cudaStream_t s,
+                                  int64_t* launches) {
+  Plan plan;
+  plan.n[0] = na; plan.n[1] = nb;
+  GK(size_scratch(plan, std::max(na, nb), s));
+  char* base = nullptr;
+  GK(reserve(wsp, carve(nullptr, plan), s, &base));
+  GeoWorkspace* ws = *wsp;
+  carve(base, plan);
   const double* set[2] = {a, b};
   for (int k = 0; k < 2; ++k) GK(build_grid(set[k], plan.n[k], plan.g[k], plan, s, launches));
   ws->plan = plan;
@@ -428,6 +601,31 @@ cudaError_t launch_geometry_queries(GeoWorkspace* ws, const double* a, const dou
     reduce_stage2_kernel<<<1, kThreads, 0, s>>>(plan.red, nv, d, out);
     *launches += 3;
   }
+  return cudaGetLastError();
+}
+
+cudaError_t launch_normals_grid(GeoWorkspace** wsp, const double* p, int64_t n, cudaStream_t s, int64_t* launches) {
+  Plan plan;
+  plan.n[0] = n;
+  GK(size_scratch(plan, n, s));
+  char* base = nullptr;
+  GK(reserve(wsp, carve_normals(nullptr, plan), s, &base));
+  carve_normals(base, plan);
+  GK(build_grid(p, n, plan.g[0], plan, s, launches));
+  (*wsp)->plan = plan;
+  return cudaSuccess;
+}
+
+cudaError_t launch_normals_query(GeoWorkspace* ws, const double* p, int64_t n, int k, double* normals, int32_t* knn, cudaStream_t s,
+                                 int64_t* launches) {
+  const Grid& g = ws->plan.g[0];
+  if (k <= 16)
+    knn_normals_kernel<16><<<blocks_for(n), kThreads, 0, s>>>(g.pts, n, k, g.params, g.starts, g.coarse, p, normals, knn);
+  else if (k <= 32)
+    knn_normals_kernel<32><<<blocks_for(n), kThreads, 0, s>>>(g.pts, n, k, g.params, g.starts, g.coarse, p, normals, knn);
+  else
+    knn_normals_kernel<64><<<blocks_for(n), kThreads, 0, s>>>(g.pts, n, k, g.params, g.starts, g.coarse, p, normals, knn);
+  *launches += 1;
   return cudaGetLastError();
 }
 

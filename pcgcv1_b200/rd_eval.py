@@ -1,7 +1,11 @@
 """Rate-distortion evaluation of one point cloud over the rate points of an ``.ini``: bits per input point against D1 / D2 PSNR.
 
     python -m pcgcv1_b200.rd_eval cloud.ply cloud_n.ply rates.ini rd.csv [--mode hyper|factorized]
-                                  [--modelname models.model_voxception] [--rates R1,R3]
+                                  [--modelname models.model_voxception] [--rates R1,R3] [--knn K]
+
+With ``--knn K`` and no file at ``cloud_n.ply``, the normals of ``cloud.ply`` are first estimated on the GPU from its K nearest
+neighbours (``pcgcv1_b200.normals``) and written to ``cloud_n.ply``; later runs, and the MPEG binary, then read that file.  Without
+``--knn``, or when the file exists, the normals file is read as given.
 
 ``rates.ini`` has the layout of the reference's rate-point files: ``[DEFAULT]`` with ``cube_size``, ``min_num`` and ``resolution``,
 then one section per rate point (``[R1]`` .. ``[Rn]``) with ``scale``, ``ckpt_dir`` and optionally ``rho_d1`` / ``rho_d2``.  For every
@@ -40,7 +44,12 @@ def parse_args(argv=None):
     ap.add_argument("--mode", default="hyper", help="entropy model: 'hyper' or 'factorized'")
     ap.add_argument("--modelname", default="models.model_voxception", help="models.model_voxception or models.model_simple")
     ap.add_argument("--rates", default="", help="comma-separated sections to evaluate ('' = every section)")
-    return ap.parse_args(argv)
+    ap.add_argument("--knn", type=int, default=None,
+                    help="when NORMALS does not exist: estimate the normals of INPUT from K nearest neighbours (1 .. 64) and write NORMALS")
+    args = ap.parse_args(argv)
+    if args.knn is not None and not 1 <= args.knn <= 64:
+        ap.error("--knn must be in 1 .. 64")
+    return args
 
 
 def _container_bytes(name, rootdir):
@@ -117,6 +126,9 @@ def main(argv=None):
         if config.getint(rate, "cube_size") != 64:
             raise SystemExit(test.CUBE_SIZE_MESSAGE)
     n_points = len(load_ply_data(args.input))
+    if args.knn is not None and not os.path.exists(args.normals):
+        from .normals import make_normals_file
+        make_normals_file(args.input, args.normals, args.knn)
     search = DeviceRhoSearch(args.input, args.normals)
     workroot = (args.csv[:-4] if args.csv.endswith(".csv") else args.csv) + "_files"
     rows = []

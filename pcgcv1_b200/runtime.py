@@ -635,6 +635,26 @@ class Codec:
                                                 normals_a.data_ptr() if normals_a is not None else None, out.data_ptr()))
         return out
 
+    def estimate_normals(self, points: torch.Tensor, k: int = 30, return_knn: bool = False):
+        """k-nearest-neighbour PCA normals of one point set on the device (pcgc_estimate_normals; contract, tie rule and sign rule
+        in include/pcgc_b200.h): points float64 [n,3] on this codec's device -> normals float64 [n,3] device tensor, and with
+        ``return_knn`` also the int32 [n,k] neighbour indices in (distance, index) order (-1 beyond n).  1 <= k <= 64.
+        Asynchronous on the current stream."""
+        if points.dtype != torch.float64 or points.dim() != 2 or points.shape[1] != 3 or points.device != self.dev \
+                or not points.is_contiguous():
+            raise ValueError("points must be a contiguous float64 [n,3] tensor on %s" % self.dev)
+        if len(points) == 0:
+            raise ValueError("estimate_normals: empty point cloud")
+        if not 1 <= int(k) <= 64:
+            raise ValueError("estimate_normals: k must be in 1 .. 64, got %s" % k)
+        k = int(k)
+        normals = torch.empty((len(points), 3), dtype=torch.float64, device=self.dev)
+        knn = torch.empty((len(points), k), dtype=torch.int32, device=self.dev) if return_knn else None
+        self._stream()
+        self._check(self.lib.pcgc_estimate_normals(self.ctx, points.data_ptr(), len(points), k, normals.data_ptr(),
+                                                   knn.data_ptr() if knn is not None else None))
+        return (normals, knn) if return_knn else normals
+
     def count_voxels(self, cubes: torch.Tensor) -> np.ndarray:
         """number of non-zero voxels per cube (np.sum(cubes, axis=(1,2,3,4)), process.py:44)."""
         B, S = cubes.shape[0], cubes.shape[1]
