@@ -52,6 +52,9 @@ typedef enum {
 
 typedef enum { PCGC_DTYPE_U8 = 0, PCGC_DTYPE_F32 = 1, PCGC_DTYPE_F64 = 2 } pcgc_dtype;
 
+/* Mesh file formats of pcgc_mesh_parse. */
+typedef enum { PCGC_MESH_OBJ = 0, PCGC_MESH_OFF = 1, PCGC_MESH_PLY = 2 } pcgc_mesh_format;
+
 /* Conv engines.  AUTO = tcgen05 implicit GEMM where a layer qualifies, FP32 CUDA-core kernel elsewhere. */
 typedef enum { PCGC_ENGINE_AUTO = 0, PCGC_ENGINE_FFMA = 1, PCGC_ENGINE_UMMA = 2 } pcgc_engine;
 
@@ -347,6 +350,45 @@ int pcgc_geometry_sums(pcgc_ctx* ctx, const double* a_dev, int64_t n_a, const do
  * Deterministic (two calls give the same bits).  Enqueued on the ctx stream, does not synchronise (except when the per-ctx
  * workspace, shared with pcgc_geometry_sums, grows). */
 int pcgc_estimate_normals(pcgc_ctx* ctx, const double* pts_dev, int64_t n, int k, double* normals_dev, int32_t* knn_idx_dev);
+
+/* ---- training data from meshes (pcgcv1_b200/dataset.py) ----------------------------------------------------------------------
+ * Triangle mesh reader.  format: PCGC_MESH_OBJ = 0, PCGC_MESH_OFF = 1, PCGC_MESH_PLY = 2.  verts: HOST float64 [vcap,3]; tris: HOST
+ * int32 [tcap,3] (0-based).  *nv / *nt are set even when PCGC_ERR_OVERFLOW reports a capacity too small; malformed input ->
+ * PCGC_ERR_CORRUPT.  Every polygon with n >= 3 corners becomes the fan (v0, v_i, v_{i+1}) in file order; a face with fewer than 3
+ * corners, an index out of range or a truncated file is PCGC_ERR_CORRUPT.
+ *   OBJ: "v x y z [w]" (further values ignored); "f" tokens i, i/j, i//k, i/j/k, negative indices counting back from the vertices
+ *        read so far, index 0 an error; vt, vn, g, o, s, usemtl, mtllib, l, p and # lines ignored, any other statement CORRUPT.
+ *   OFF: "OFF" or "COFF" header (the counts may be glued on: "OFF490 518 0"), # comments, "nv nf ne", vertex lines "x y z ..."
+ *        (values after z ignored), face lines "n i0 .. i{n-1} ..." (colour values after the indices ignored).
+ *   PLY: "ascii 1.0" or "binary_little_endian 1.0" (any other format: PCGC_ERR_BAD_ARG); element vertex with x / y / z of any
+ *        scalar type (other properties skipped), element face with "property list <count> <index> vertex_indices|vertex_index"
+ *        (other properties skipped); other elements skipped, in binary files only when all their properties are scalars. */
+int pcgc_mesh_parse(const char* data, int64_t nbytes, int format, double* verts, int64_t vcap, int32_t* tris, int64_t tcap,
+                    int64_t* nv, int64_t* nt);
+
+/* Uniform surface sampling of a triangle mesh, grid quantisation and deduplication.  verts_dev float64 [nv,3], tris_dev int32 [nt,3],
+ * points_dev int32 [n,3] (out), samples_dev float64 [n,3] and face_dev int32 [n] (optional outputs, NULL = not written): DEVICE
+ * pointers; rot_host float64 [9] (row-major R) and *n_unique: HOST.  This project's own exact rule (no external sampler's):
+ *   1. FACE WEIGHT: e1 = B - A, e2 = C - A, c = e1 x e2 component-wise (cx = e1y*e2z - e1z*e2y, ...), a2 = sqrt((cx*cx + cy*cy) + cz*cz)
+ *      (twice the area).  With M = max a2 and frexp(M) = (m, e): w = (uint64) floor(ldexp(a2, 32 - e)) < 2^32 (exact scaling).
+ *      w = 0 exactly when a2 < 2^(e-32): every degenerate face and every face below 2^-32 of the largest (faces up to 2^-31 of the
+ *      largest may fall under it too) is NEVER drawn.  P = exclusive prefix sum of w (uint64, exact), W = total.
+ *   2. SAMPLE j (0 <= j < n): r = philox4x32_10(counter (j_lo, j_hi), key (seed_lo, seed_hi)); t = r1 * 2^32 + r0;
+ *      target = mulhi64(t, W); face f = the largest f with P[f] <= target.  u1 = (r2 + 0.5) 2^-32, u2 = (r3 + 0.5) 2^-32, s = sqrt(u1),
+ *      a = 1 - s, b = s*(1 - u2), c = s*u2; p = (a*A + b*B) + c*C per coordinate (uniform density on the triangle).
+ *   3. ROTATION AND GRID: q = R p, row r = (R[r][0]*p0 + R[r][1]*p1) + R[r][2]*p2.  [lo, hi] = box of the rotated vertices that a
+ *      face references (unreferenced vertices are ignored; the box depends only on the mesh and R, not on n or the seed);
+ *      E = max over axes of (hi - lo), scale = (resolution - 1) / E; g = clamp(rint((q - lo) * scale), 0, resolution - 1), rint
+ *      rounding half to even.
+ *   4. DEDUPLICATION: key (gx*R + gy)*R + gz (R = resolution), radix-sorted over 3*ceil(log2 R) bits, unique.  points_dev[0 .. *n_unique)
+ *      = the distinct grid points in ascending key order (lexicographic (x, y, z)); samples_dev = q and face_dev = f in sample order.
+ * Every multiply and add is rounded on its own (no FMA).  PCGC_ERR_BAD_ARG: 2 <= resolution <= 4096, 1 <= n <= 2^28,
+ * 1 <= nt <= 2^30, 1 <= nv < 2^31 violated; a face index outside [0, nv); a non-finite a2; W == 0; a zero or non-finite box extent E
+ * (the last four detected on the device).  Runs on the ctx stream and synchronises once (n_unique and the error flags); the per-ctx
+ * workspace grows as needed.  Deterministic: two calls give the same bits. */
+int pcgc_mesh_sample(pcgc_ctx* ctx, const double* verts_dev, int64_t nv, const int32_t* tris_dev, int64_t nt, const double* rot_host,
+                     int64_t n, uint64_t seed, int resolution, int32_t* points_dev, int64_t* n_unique, double* samples_dev,
+                     int32_t* face_dev);
 
 #ifdef __cplusplus
 }

@@ -17,6 +17,7 @@ LIB_PATH = os.environ.get("PCGC_LIB") or os.path.join(_HERE, "libpcgc_b200.so") 
 # enums of include/pcgc_b200.h
 NET_VOX_ANALYSIS, NET_VOX_SYNTHESIS, NET_HYPER_ENCODER, NET_HYPER_DECODER, NET_SIMPLE_ANALYSIS, NET_SIMPLE_SYNTHESIS = range(6)
 DTYPE_U8, DTYPE_F32, DTYPE_F64 = range(3)
+MESH_OBJ, MESH_OFF, MESH_PLY = range(3)
 ENGINE_AUTO, ENGINE_FFMA, ENGINE_UMMA = range(3)
 MAX_SYMBOLS = 64
 ERR_BAD_ARG, ERR_BAD_RANGE, ERR_CUDA, ERR_OOM, ERR_NOT_READY, ERR_OVERFLOW, ERR_CORRUPT = -1, -2, -3, -4, -5, -6, -7
@@ -93,6 +94,8 @@ SIGNATURES = {
     "pcgc_extract_points": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i64, _vp]),
     "pcgc_geometry_sums": (_i, [_vp, _vp, _i64, _vp, _i64, _vp, _vp]),
     "pcgc_estimate_normals": (_i, [_vp, _vp, _i64, _i, _vp, _vp]),
+    "pcgc_mesh_parse": (_i, [_vp, _i64, _i, _vp, _i64, _vp, _i64, C.POINTER(_i64), C.POINTER(_i64)]),
+    "pcgc_mesh_sample": (_i, [_vp, _vp, _i64, _vp, _i64, _vp, _i64, C.c_uint64, _i, _vp, C.POINTER(_i64), _vp, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None

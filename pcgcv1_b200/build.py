@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "_obj")
 LIB = os.path.join(HERE, "libpcgc_b200.so")
-SOURCES = ["api.cu", "conv_ffma.cu", "umma_conv.cu", "umma_win.cu", "entropy.cu", "gpu_coder.cu", "train.cu", "topk.cu", "voxelize.cu", "metrics.cu", "coder.cpp", "pointio.cpp"]
+SOURCES = ["api.cu", "conv_ffma.cu", "umma_conv.cu", "umma_win.cu", "entropy.cu", "gpu_coder.cu", "train.cu", "topk.cu", "voxelize.cu", "metrics.cu", "meshsample.cu", "coder.cpp", "pointio.cpp", "meshio.cpp"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC,-O3,-Wall,-Wno-unused-function,-ffp-contract=off", "--expt-relaxed-constexpr"]
@@ -31,8 +31,10 @@ def _deps_mtime() -> float:
 
 # entropy.cu holds the device copy of the likelihood -> integer CDF path (det_math.h, cdf_norm.h) whose results must equal the host
 # copy's bit for bit: no mul+add contraction there (the host objects are built with -ffp-contract=off).
-# metrics.cu computes the per-point D1 / D2 values in NumPy's arithmetic (every multiply and add rounded on its own).
-PER_FILE = {"entropy.cu": ["-fmad=false"] + os.environ.get("PCGC_ENTROPY_FLAGS", "").split(), "metrics.cu": ["-fmad=false"]}
+# metrics.cu computes the per-point D1 / D2 values in NumPy's arithmetic (every multiply and add rounded on its own); so does
+# meshsample.cu for the face weights, the sample points and their grid cells, which a NumPy restatement reproduces bit for bit.
+PER_FILE = {"entropy.cu": ["-fmad=false"] + os.environ.get("PCGC_ENTROPY_FLAGS", "").split(), "metrics.cu": ["-fmad=false"],
+            "meshsample.cu": ["-fmad=false"]}
 
 
 def _compile(src: str, verbose: bool) -> str:

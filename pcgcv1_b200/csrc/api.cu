@@ -216,6 +216,7 @@ struct pcgc_ctx {
   int64_t* off_dev = nullptr; size_t off_cap = 0;
   int64_t* chunk_dev = nullptr; size_t chunk_cap = 0;   // voxelize / extract workspace
   GeoWorkspace* geo_ws = nullptr;   // pcgc_geometry_sums (metrics.cu)
+  MeshWorkspace* mesh_ws = nullptr; // pcgc_mesh_sample (meshsample.cu)
   // far-field tiles of the analysis transform (PCGC_FARFIELD; DESIGN 4.1): the three VRN-16 block outputs of the all-zero cube, the
   // classification masks of the current sub-batch
   uint8_t* ff_zero = nullptr; float* ff_y = nullptr;
@@ -951,6 +952,7 @@ float* ctx_workspace(pcgc_ctx* c, int slot, size_t floats) {
 }
 void ctx_prof_begin(pcgc_ctx* c, const char* tag, double flops, double bytes) { prof_begin(c, tag, flops, bytes); }
 void ctx_prof_end(pcgc_ctx* c) { prof_end(c); }
+MeshWorkspace** ctx_mesh_workspace(pcgc_ctx* c) { return &c->mesh_ws; }
 }  // namespace pcgc
 
 extern "C" {
@@ -1004,6 +1006,7 @@ void pcgc_destroy(pcgc_ctx* ctx) {
     }
   for (auto& b : ctx->bn) if (b.params) cudaFree(b.params);
   free_geometry_workspace(ctx->geo_ws);
+  free_mesh_workspace(ctx->mesh_ws);
   if (ctx->ff_zero) cudaFree(ctx->ff_zero);
   if (ctx->ff_y) cudaFree(ctx->ff_y);
   for (auto e : ctx->ff_e) if (e) cudaFree(e);

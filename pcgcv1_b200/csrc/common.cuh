@@ -144,4 +144,9 @@ cudaError_t launch_normals_grid(GeoWorkspace** ws, const double* p, int64_t n, c
 cudaError_t launch_normals_query(GeoWorkspace* ws, const double* p, int64_t n, int k, double* normals, int32_t* knn, cudaStream_t s,
                                  int64_t* launches);
 
+// meshsample.cu: the per-ctx workspace of pcgc_mesh_sample (grown on demand, freed with the ctx)
+struct MeshWorkspace;
+MeshWorkspace** ctx_mesh_workspace(pcgc_ctx* c);
+void free_mesh_workspace(MeshWorkspace* ws);
+
 }  // namespace pcgc

@@ -655,6 +655,42 @@ class Codec:
                                                    knn.data_ptr() if knn is not None else None))
         return (normals, knn) if return_knn else normals
 
+    def sample_mesh(self, verts: torch.Tensor, tris: torch.Tensor, n: int, seed: int, resolution: int, rotation=None,
+                    return_samples: bool = False):
+        """Uniform surface samples of a triangle mesh on a grid, deduplicated (pcgc_mesh_sample; the exact rule is in
+        include/pcgc_b200.h): verts float64 [V,3] and tris int32 [F,3] on this codec's device, ``n`` samples drawn with ``seed``,
+        rotated by ``rotation`` (float64 [3,3]; None = identity), on a ``resolution``^3 grid -> the distinct grid points as an int32
+        [m,3] device tensor in lexicographic order, and with ``return_samples`` also the rotated samples float64 [n,3] and their
+        faces int32 [n] in sample order.  Synchronises once."""
+        if verts.dtype != torch.float64 or verts.dim() != 2 or verts.shape[1] != 3 or verts.device != self.dev \
+                or not verts.is_contiguous():
+            raise ValueError("verts must be a contiguous float64 [V,3] tensor on %s" % self.dev)
+        if tris.dtype != torch.int32 or tris.dim() != 2 or tris.shape[1] != 3 or tris.device != self.dev or not tris.is_contiguous():
+            raise ValueError("tris must be a contiguous int32 [F,3] tensor on %s" % self.dev)
+        if len(verts) == 0 or len(tris) == 0:
+            raise ValueError("sample_mesh: the mesh has no vertices or no faces")
+        if not 1 <= int(n) <= 2 ** 28:
+            raise ValueError("sample_mesh: n must be in 1 .. 2^28, got %s" % n)
+        if not 2 <= int(resolution) <= 4096:
+            raise ValueError("sample_mesh: resolution must be in 2 .. 4096, got %s" % resolution)
+        if not 0 <= int(seed) < 2 ** 64:
+            raise ValueError("sample_mesh: seed must be in 0 .. 2^64 - 1, got %s" % seed)
+        rot = np.eye(3) if rotation is None else np.ascontiguousarray(rotation, dtype=np.float64)
+        if rot.shape != (3, 3) or not np.all(np.isfinite(rot)):
+            raise ValueError("sample_mesh: rotation must be a finite [3,3] matrix")
+        n = int(n)
+        points = torch.empty((n, 3), dtype=torch.int32, device=self.dev)
+        samples = torch.empty((n, 3), dtype=torch.float64, device=self.dev) if return_samples else None
+        faces = torch.empty(n, dtype=torch.int32, device=self.dev) if return_samples else None
+        m = C.c_int64()
+        self._stream()
+        self._check(self.lib.pcgc_mesh_sample(self.ctx, verts.data_ptr(), len(verts), tris.data_ptr(), len(tris), rot.ctypes.data, n,
+                                              int(seed), int(resolution), points.data_ptr(), C.byref(m),
+                                              samples.data_ptr() if return_samples else None,
+                                              faces.data_ptr() if return_samples else None))
+        points = points[:m.value]
+        return (points, samples, faces) if return_samples else points
+
     def count_voxels(self, cubes: torch.Tensor) -> np.ndarray:
         """number of non-zero voxels per cube (np.sum(cubes, axis=(1,2,3,4)), process.py:44)."""
         B, S = cubes.shape[0], cubes.shape[1]

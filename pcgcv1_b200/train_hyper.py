@@ -6,6 +6,8 @@ What the reference's loop does, and where it is here:
 * data (``:121-122,171-177``): a directory of per-cube point files (``h5py.File(f)['data']``: integer [n,3] points of one 64^3
   cube), ``random.sample(train_list, BATCH_SIZE)`` per step with ``random.seed(3)`` (``:17``), the first ``1/RATIO_EVAL`` of the
   file list held out for evaluation -> ``CubeFiles`` (h5 when h5py is importable, .npy / .npz otherwise; same sampling).
+  ``python -m pcgcv1_b200.dataset`` writes such files from meshes (OBJ / OFF / PLY; the reference's ``generate_dataset.py`` and
+  ``dataprocess/mesh2pc.py``).
 * the step (``:179-214``) -> ``HyperTrainer.train_step`` (seeded Philox noise: step number = seed).
 * running means of bpp / IoU every DISPLAY_STEP (``:216-248``): ``select_voxels`` of the reconstruction with the TRUE point count
   of every cube, then ``get_classify_metrics`` (``loss.py:60-78``) -> ``iou`` below.
