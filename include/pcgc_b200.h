@@ -255,9 +255,22 @@ int pcgc_train_conv_forward(pcgc_ctx* ctx, const float* x, int B, int n, int cin
 /* dx [B,n,n,n,cin] from the output gradient g [B,m,m,m,cout] of the same layer (n = the layer's INPUT grid). */
 int pcgc_train_conv_dgrad(pcgc_ctx* ctx, const float* g, int B, int n, int cin, int cout, int k, int stride, int transposed,
                           const float* w_keras, float* dx);
-/* dw (the layer's Keras layout) and db [cout] (NULL for use_bias=False layers) from the layer input x and g. */
+/* dw (the layer's Keras layout) and db [cout] (NULL for use_bias=False layers) from the layer input x and g.
+ * The form of dW follows from the shape alone.  k <= 3 (every Voxception layer): the tile kernel, one partial per anchor tile
+ * (2x4x4 anchors at stride 2, 4x8x8 at stride 1), summed in groups of 64 tiles and then over the groups; the workspace grows with
+ * the batch; also k = 5, where it measured faster than the slice kernel.  k = 9 with <= 64 anchor channels (the anchor side is g
+ * for a conv, x for a transposed conv; conv_1 and deconv_3 of model_simple): the slice kernel.  Its anchor tiles (2x4x8) are cut
+ * into S contiguous runs, S = min(128, ceil(592 / Y)) with Y = ceil(min(cg, 8) * ceil(ca / 4) * k^2 / 128) * ceil(cg / 8) (cg = the other side's channels), a function of the shape only;
+ * every dW element is summed over the tiles of a run in increasing order (voxels in z, y, x order within a tile), then over the
+ * runs in increasing order.  Its workspace is S * k^3 * cin * cout floats <= 128 * k^3 * cin * cout, whatever the batch.
+ * Neither form uses atomics: two calls return the same bits. */
 int pcgc_train_conv_wgrad(pcgc_ctx* ctx, const float* x, const float* g, int B, int n, int cin, int cout, int k, int stride,
                           int transposed, float* dw, float* db);
+/* pcgc_train_conv_wgrad with the dW form forced: 0 = tile kernel (any odd k), 1 = slice kernel (k in {3, 5, 9}, <= 64 anchor
+ * channels, else PCGC_ERR_BAD_ARG).  *partial_floats (nullable) = the size of the partial buffer the form used.  Test / benchmark
+ * hook: the product path never calls it. */
+int pcgc_debug_train_wgrad(pcgc_ctx* ctx, int form, const float* x, const float* g, int B, int n, int cin, int cout, int k, int stride,
+                           int transposed, float* dw, float* db, int64_t* partial_floats);
 /* out = g where y > 0 else 0 (gradient through a fused ReLU; y = the layer output). */
 int pcgc_train_relu_backward(pcgc_ctx* ctx, const float* g, const float* y, int64_t n, float* out);
 /* _VoxceptionResNet merge (model_voxception.py:64-67): out = relu(x + concat[t12, t23]) over nvox voxels of c channels. */

@@ -73,6 +73,7 @@ SIGNATURES = {
     "pcgc_train_conv_forward": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _i, _vp]),
     "pcgc_train_conv_dgrad": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     "pcgc_train_conv_wgrad": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
+    "pcgc_debug_train_wgrad": (_i, [_vp, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, C.POINTER(_i64)]),
     "pcgc_train_relu_backward": (_i, [_vp, _vp, _vp, _i64, _vp]),
     "pcgc_train_vrn_merge": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _vp]),
     "pcgc_train_vrn_merge_backward": (_i, [_vp, _vp, _vp, _i64, _i, _vp, _vp, _vp]),

@@ -11,7 +11,8 @@
 //     device per call (they change every step).
 //   * weight-gradient: dW[tap][cg][ca] = sum_v T[s*v + tap - pad][cg] * A[v][ca] over anchor voxels v (A = output gradient for a
 //     conv, = input for a transposed conv; T = the other one), computed as fixed-order partial sums over voxel ranges and a
-//     second fixed-order pass over the partials (no atomics).
+//     second fixed-order pass over the partials (no atomics): per anchor tile for k <= 3 (wgrad_tile_kernel), per fixed run of
+//     tiles for the k = 9 layers of model_simple (wgrad_slice_kernel).
 #include <math.h>
 #include <stdint.h>
 
@@ -189,6 +190,101 @@ wgrad_tile_kernel(const float* __restrict__ T, const float* __restrict__ A, int 
     if (left > 1) o[1] = acc1;
     if (left > 2) o[2] = acc2;
     if (left > 3) o[3] = acc3;
+  }
+}
+
+// The same dW for the 9^3 layers of model_simple (conv_1, deconv_3: SURVEY.md 8d).  The tile kernel above writes one partial per
+// anchor tile (764 MB for conv_1 at batch 8) and stages 16 gathered channels even when the layer has one.  Here:
+//   * the anchor tiles (2x4x8 voxels) are cut into `slices` contiguous runs; a block owns one run and a fixed set of units, keeps
+//     its accumulators in registers across the run and writes ONE partial per slice: partial[slice][tap][cg][ca].  The slice
+//     count is a function of the layer shape only, so the workspace does not grow with the batch;
+//   * a unit = (gathered channel, quad of anchor channels, kz, ky) with all k kx-taps: per row of 8 anchor voxels it loads the
+//     (8-1)*S + k gathered values of the row once and 8 float4 of A, for 8 * k * 4 FMAs;
+//   * only the channels that exist are staged: at most 8 gathered channels (a 1-channel side stages 1) and ceil(ca/4) quads.
+// Accumulation order of every dW element: tiles of the slice in increasing order, voxels of a tile in (z, y, x) order, then the
+// slices in increasing order (reduce_rows_kernel).  No atomics: two calls return the same bits.
+constexpr int WGL_TZ = 2, WGL_TY = 4, WGL_TX = 8, WGL_GN = 8, WGL_THREADS = 128, WGL_MAX_SLICES = 128;
+
+template <int K, int S>
+__global__ void __launch_bounds__(WGL_THREADS)
+wgrad_slice_kernel(const float* __restrict__ T, const float* __restrict__ A, int B, int na, int nt, int cg, int ca, int pad, int slices,
+                   int ychunks, float* __restrict__ partial) {
+  constexpr int TZ = WGL_TZ, TY = WGL_TY, TX = WGL_TX, NV = TZ * TY * TX;
+  constexpr int BZ = (TZ - 1) * S + K, BY = (TY - 1) * S + K, BX = (TX - 1) * S + K, NB = BZ * BY * BX;
+  constexpr int ROW = (TX - 1) * S + K;
+  extern __shared__ float4 sm4[];
+  const int quads = (ca + 3) >> 2, cap = quads * 4;
+  float* sA = reinterpret_cast<float*>(sm4);                 // [NV][cap]
+  const int chunk = blockIdx.y / ychunks;
+  const int g0 = chunk * WGL_GN, gn = min(WGL_GN, cg - g0);
+  float* sT = sA + NV * cap;                                 // [NB][gn]
+  const int u = (blockIdx.y % ychunks) * WGL_THREADS + threadIdx.x;
+  const bool active = u < gn * quads * K * K;
+  const int c = u % gn, q = (u / gn) % quads, kzy = u / (gn * quads);
+  const int kz = kzy / K, ky = kzy % K;
+  const int tiles_x = na / TX, tiles_y = na / TY, tiles_z = na / TZ;
+  const long long tiles = (long long)B * tiles_z * tiles_y * tiles_x;
+  const long long t0 = tiles * blockIdx.x / slices, t1 = tiles * (blockIdx.x + 1) / slices;
+  float acc[K][4];
+#pragma unroll
+  for (int j = 0; j < K; ++j) acc[j][0] = acc[j][1] = acc[j][2] = acc[j][3] = 0.f;
+  for (long long tile = t0; tile < t1; ++tile) {
+    long long t = tile;
+    const int bx = (int)(t % tiles_x); t /= tiles_x;
+    const int by = (int)(t % tiles_y); t /= tiles_y;
+    const int bz = (int)(t % tiles_z); const int b = (int)(t / tiles_z);
+    const int z0 = bz * TZ, y0 = by * TY, x0 = bx * TX;
+    __syncthreads();                                         // the previous tile's readers are done
+    for (int i = threadIdx.x; i < NV * cap; i += WGL_THREADS) {
+      const int ch = i % cap, v = i / cap;
+      const int x = v % TX, y = (v / TX) % TY, z = v / (TX * TY);
+      float val = 0.f;
+      if (ch < ca) val = __ldg(A + ((((size_t)b * na + z0 + z) * na + y0 + y) * na + x0 + x) * ca + ch);
+      sA[i] = val;
+    }
+    for (int i = threadIdx.x; i < NB * gn; i += WGL_THREADS) {
+      const int ch = i % gn, v = i / gn;
+      const int x = v % BX, y = (v / BX) % BY, z = v / (BX * BY);
+      const int gz = z0 * S - pad + z, gy = y0 * S - pad + y, gx = x0 * S - pad + x;
+      float val = 0.f;
+      if ((unsigned)gz < (unsigned)nt && (unsigned)gy < (unsigned)nt && (unsigned)gx < (unsigned)nt)
+        val = __ldg(T + ((((size_t)b * nt + gz) * nt + gy) * nt + gx) * cg + g0 + ch);
+      sT[i] = val;
+    }
+    __syncthreads();
+    if (active) {
+#pragma unroll 1
+      for (int z = 0; z < TZ; ++z)
+#pragma unroll 1
+        for (int y = 0; y < TY; ++y) {
+          const float* tr = sT + ((size_t)((z * S + kz) * BY + y * S + ky) * BX) * gn + c;
+          float tv[ROW];
+#pragma unroll
+          for (int i = 0; i < ROW; ++i) tv[i] = tr[i * gn];
+          const float4* ar = reinterpret_cast<const float4*>(sA + (size_t)(z * TY + y) * TX * cap) + q;
+#pragma unroll
+          for (int x = 0; x < TX; ++x) {
+            const float4 a4 = ar[x * quads];
+#pragma unroll
+            for (int kx = 0; kx < K; ++kx) {
+              const float tt = tv[x * S + kx];
+              acc[kx][0] = fmaf(tt, a4.x, acc[kx][0]); acc[kx][1] = fmaf(tt, a4.y, acc[kx][1]);
+              acc[kx][2] = fmaf(tt, a4.z, acc[kx][2]); acc[kx][3] = fmaf(tt, a4.w, acc[kx][3]);
+            }
+          }
+        }
+    }
+  }
+  if (!active) return;
+  const int left = ca - 4 * q;
+  float* out = partial + (size_t)blockIdx.x * K * K * K * cg * ca;
+#pragma unroll
+  for (int kx = 0; kx < K; ++kx) {
+    float* o = out + ((size_t)(kzy * K + kx) * cg + g0 + c) * ca + 4 * q;
+    o[0] = acc[kx][0];
+    if (left > 1) o[1] = acc[kx][1];
+    if (left > 2) o[2] = acc[kx][2];
+    if (left > 3) o[3] = acc[kx][3];
   }
 }
 
@@ -548,42 +644,89 @@ int pcgc_train_conv_dgrad(pcgc_ctx* ctx, const float* g, int B, int n, int cin, 
   return r;
 }
 
-/* dw (Keras layout of the layer) and db (nullable) from the layer input x [B,n^3,cin] and the output gradient g. */
-int pcgc_train_conv_wgrad(pcgc_ctx* ctx, const float* x, const float* g, int B, int n, int cin, int cout, int k, int stride,
-                          int transposed, float* dw, float* db) {
-  if (!ctx || !x || !g || !dw || B < 1) return PCGC_ERR_BAD_ARG;
+}  // extern "C"
+
+namespace {
+
+// The slice form takes k in {3, 5, 9} (the model's extents) and up to 64 anchor channels (the staged A tile).
+bool slice_form_supported(int k, int ca) { return (k == 3 || k == 5 || k == 9) && ca >= 1 && ca <= 64; }
+
+// Slice count of the slice form: enough blocks for ~4 per SM, from the layer shape only (never from the batch).
+int slice_count(int k, int cg, int ca, int* ychunks) {
+  const int quads = (ca + 3) / 4, gmax = std::min(cg, WGL_GN);
+  *ychunks = (gmax * quads * k * k + WGL_THREADS - 1) / WGL_THREADS;
+  const int ys = *ychunks * ((cg + WGL_GN - 1) / WGL_GN);
+  return std::max(1, std::min(WGL_MAX_SLICES, (148 * 4 + ys - 1) / ys));
+}
+
+template <int K, int S>
+cudaError_t launch_slice(dim3 grid, size_t smem, cudaStream_t s, const float* T, const float* A, int B, int na, int nt, int cg, int ca,
+                         int pad, int slices, int ychunks, float* partial) {
+  cudaError_t e = cudaFuncSetAttribute(wgrad_slice_kernel<K, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  wgrad_slice_kernel<K, S><<<grid, WGL_THREADS, smem, s>>>(T, A, B, na, nt, cg, ca, pad, slices, ychunks, partial);
+  return cudaGetLastError();
+}
+
+// dW (and db when non-null) of one layer by the given form (0 = tile kernel, 1 = slice kernel); *partial_floats (nullable) = the
+// size of the partial buffer the form used.
+int wgrad_run(pcgc_ctx* ctx, int form, const float* x, const float* g, int B, int n, int cin, int cout, int k, int stride, int transposed,
+              float* dw, float* db, int64_t* partial_floats) {
   cudaStream_t s = ctx_stream(ctx);
   // anchor grid / tensors: conv: A = g (n/stride, cout), T = x (n, cin), dW[tap][cin][cout];  convT: A = x (n, cin), T = g (n*stride, cout), dW[tap][cout][cin]
   const int na = transposed ? n : n / stride, nt = transposed ? n * stride : n;
   const int ca = transposed ? cin : cout, cg = transposed ? cout : cin;
   const float* A = transposed ? x : g; const float* T = transposed ? g : x;
-  const int taps = k * k * k, pairs = cg * ca;
+  const int taps = k * k * k, pairs = cg * ca, total = taps * pairs;
   const long long va = (long long)B * na * na * na;
   if ((stride != 1 && stride != 2) || na % 8 != 0) return ctx_fail(ctx, PCGC_ERR_BAD_ARG, "train wgrad: stride 1 or 2 and an anchor grid multiple of 8");
-  const int tz = stride == 1 ? 4 : 2, ty = stride == 1 ? 8 : 4, tx = stride == 1 ? 8 : 4;
-  const int tiles = B * (na / tz) * (na / ty) * (na / tx);
-  float* partial = ctx_workspace(ctx, 1, (size_t)tiles * taps * pairs + 64);
-  if (!partial) return ctx_fail(ctx, PCGC_ERR_OOM, "train: wgrad workspace");
-  const size_t brick = (size_t)((tz - 1) * stride + k) * ((ty - 1) * stride + k) * ((tx - 1) * stride + k);
-  const size_t smem = (brick * 16 + (size_t)tz * ty * tx * 16) * sizeof(float);
-  ctx_prof_begin(ctx, "train_conv_wgrad", 2.0 * va * taps * pairs, 0);
-  const dim3 grid(tiles, (cg + 15) / 16, (ca + 15) / 16);
-  if (stride == 1) {
-    TCK(cudaFuncSetAttribute(wgrad_tile_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    wgrad_tile_kernel<1><<<grid, 256, smem, s>>>(T, A, na, nt, cg, ca, k, pad_before(k, stride), partial);
+  if (form == 1 && !slice_form_supported(k, ca)) return ctx_fail(ctx, PCGC_ERR_BAD_ARG, "train wgrad: the slice form takes k in {3,5,9} and <= 64 anchor channels");
+  int64_t rows;                                                      // partial rows the fixed-order passes sum
+  if (form == 1) {
+    int ychunks;
+    const int slices = slice_count(k, cg, ca, &ychunks);
+    float* partial = ctx_workspace(ctx, 1, (size_t)slices * total + 64);
+    if (!partial) return ctx_fail(ctx, PCGC_ERR_OOM, "train: wgrad workspace");
+    constexpr int NV = WGL_TZ * WGL_TY * WGL_TX;
+    const size_t brick = (size_t)((WGL_TZ - 1) * stride + k) * ((WGL_TY - 1) * stride + k) * ((WGL_TX - 1) * stride + k);
+    const size_t smem = ((size_t)NV * ((ca + 3) & ~3) + brick * std::min(cg, WGL_GN)) * sizeof(float);
+    const dim3 grid(slices, ychunks * ((cg + WGL_GN - 1) / WGL_GN));
+    const int pad = pad_before(k, stride);
+    ctx_prof_begin(ctx, "train_conv_wgrad_large", 2.0 * va * taps * pairs, 0);
+    cudaError_t e;
+#define PCGC_SLICE(KV, SV) e = launch_slice<KV, SV>(grid, smem, s, T, A, B, na, nt, cg, ca, pad, slices, ychunks, partial)
+    if (stride == 1) { if (k == 3) PCGC_SLICE(3, 1); else if (k == 5) PCGC_SLICE(5, 1); else PCGC_SLICE(9, 1); }
+    else { if (k == 3) PCGC_SLICE(3, 2); else if (k == 5) PCGC_SLICE(5, 2); else PCGC_SLICE(9, 2); }
+#undef PCGC_SLICE
+    TCK(e);
+    reduce_rows_kernel<<<dim3((total + 255) / 256, 1), 256, 0, s>>>(partial, slices, total, slices, dw);
+    *ctx_launches(ctx) += 2;
+    rows = slices;
   } else {
-    TCK(cudaFuncSetAttribute(wgrad_tile_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    wgrad_tile_kernel<2><<<grid, 256, smem, s>>>(T, A, na, nt, cg, ca, k, pad_before(k, stride), partial);
-  }
-  {
+    const int tz = stride == 1 ? 4 : 2, ty = stride == 1 ? 8 : 4, tx = stride == 1 ? 8 : 4;
+    const int tiles = B * (na / tz) * (na / ty) * (na / tx);
+    float* partial = ctx_workspace(ctx, 1, (size_t)tiles * taps * pairs + 64);
+    if (!partial) return ctx_fail(ctx, PCGC_ERR_OOM, "train: wgrad workspace");
+    const size_t brick = (size_t)((tz - 1) * stride + k) * ((ty - 1) * stride + k) * ((tx - 1) * stride + k);
+    const size_t smem = (brick * 16 + (size_t)tz * ty * tx * 16) * sizeof(float);
+    ctx_prof_begin(ctx, "train_conv_wgrad", 2.0 * va * taps * pairs, 0);
+    const dim3 grid(tiles, (cg + 15) / 16, (ca + 15) / 16);
+    if (stride == 1) {
+      TCK(cudaFuncSetAttribute(wgrad_tile_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      wgrad_tile_kernel<1><<<grid, 256, smem, s>>>(T, A, na, nt, cg, ca, k, pad_before(k, stride), partial);
+    } else {
+      TCK(cudaFuncSetAttribute(wgrad_tile_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      wgrad_tile_kernel<2><<<grid, 256, smem, s>>>(T, A, na, nt, cg, ca, k, pad_before(k, stride), partial);
+    }
     // fixed-order two-level sum over the tiles: groups of 64 tiles, then the group sums
-    const int total = taps * pairs, group = 64, ngrp = (tiles + group - 1) / group;
+    const int group = 64, ngrp = (tiles + group - 1) / group;
     float* p2 = ctx_workspace(ctx, 2, (size_t)ngrp * total + (size_t)64 * 64 + 64);
     if (!p2) return ctx_fail(ctx, PCGC_ERR_OOM, "train: wgrad reduce workspace");
     reduce_rows_kernel<<<dim3((total + 255) / 256, ngrp), 256, 0, s>>>(partial, tiles, total, group, p2);
     reduce_rows_kernel<<<dim3((total + 255) / 256, 1), 256, 0, s>>>(p2, ngrp, total, ngrp, dw);
+    *ctx_launches(ctx) += 3;
+    rows = tiles;
   }
-  *ctx_launches(ctx) += 3;
   if (db) {
     const int no = transposed ? n * stride : n / stride;
     const long long vo = (long long)B * no * no * no;
@@ -597,7 +740,30 @@ int pcgc_train_conv_wgrad(pcgc_ctx* ctx, const float* x, const float* g, int B, 
   }
   ctx_prof_end(ctx);
   TCK(cudaGetLastError());
+  if (partial_floats) *partial_floats = rows * total;
   return PCGC_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+/* dw (Keras layout of the layer) and db (nullable) from the layer input x [B,n^3,cin] and the output gradient g. */
+int pcgc_train_conv_wgrad(pcgc_ctx* ctx, const float* x, const float* g, int B, int n, int cin, int cout, int k, int stride,
+                          int transposed, float* dw, float* db) {
+  if (!ctx || !x || !g || !dw || B < 1) return PCGC_ERR_BAD_ARG;
+  // The slice kernel for k = 9 (conv_1 / deconv_3 of model_simple: 1.16 ms against 6.06 ms for the tile kernel at batch 8 on a
+  // B200); every other layer keeps the tile kernel -- k <= 3 (every Voxception layer) and k = 5, where the tile kernel measured
+  // faster (conv_2 / deconv_2: 0.92 ms against 3.18 ms).
+  const int form = k == 9 && slice_form_supported(k, transposed ? cin : cout) ? 1 : 0;
+  return wgrad_run(ctx, form, x, g, B, n, cin, cout, k, stride, transposed, dw, db, nullptr);
+}
+
+/* pcgc_train_conv_wgrad with the dW form forced (0 = tile kernel, 1 = slice kernel), for tests and benchmarks. */
+int pcgc_debug_train_wgrad(pcgc_ctx* ctx, int form, const float* x, const float* g, int B, int n, int cin, int cout, int k, int stride,
+                           int transposed, float* dw, float* db, int64_t* partial_floats) {
+  if (!ctx || !x || !g || !dw || B < 1 || (form != 0 && form != 1)) return PCGC_ERR_BAD_ARG;
+  return wgrad_run(ctx, form, x, g, B, n, cin, cout, k, stride, transposed, dw, db, partial_floats);
 }
 
 int pcgc_train_relu_backward(pcgc_ctx* ctx, const float* g, const float* y, int64_t n, float* out) {

@@ -24,6 +24,9 @@ TensorBoard summaries (``tf.contrib.summary``) become one JSON line per display 
 The rho search of ``eval_ablation_studies.py:152-205`` needs the external ``pc_error`` binary and is not built.
 
 ``python -m pcgcv1_b200.train_hyper --data 'points64/*.h5' --alpha 0.75 --beta 3 --num_iteration 300000``
+
+The factorized-prior models (``model_simple`` and the Voxception transforms without the hyperprior) train with the same loop
+(``run_loop``): ``python -m pcgcv1_b200.train_factorized`` (pcgcv1_b200/train_factorized.py).
 """
 from __future__ import annotations
 
@@ -174,13 +177,15 @@ def evaluate(weights, files: Sequence[str], batch_size: int = 8, device: Optiona
 
 
 # ------------------------------------------------------------------------------------------- loop
-def train(files: Sequence[str], ckpt_dir: str, alpha=2.0, beta=3.0, gamma=1.0, delta=1.0, lr=1e-5, num_iteration=int(3e5), batch_size=8,
-          init_ckpt_dir: str = "", reset_optimizer: int = 0, lower_bound: float = 1e-9, display_step: int = DISPLAY_STEP,
-          save_step: int = SAVE_STEP, eval_cubes: int = 256, log=print, distortion: str = "bce"):
-    """``train()`` of train_hyper.py:165-266.  Returns the trainer (rank-local)."""
+def run_loop(files: Sequence[str], ckpt_dir: str, model: str, make_trainer, evaluate_fn, rate_keys: Sequence[str], num_iteration: int,
+             batch_size: int, init_ckpt_dir: str, reset_optimizer: int, display_step: int, save_step: int, eval_cubes: int, log):
+    """The loop both training commands share (train_hyper.py:165-266): resume / seeding, seeded sampling, one ``train_step`` per
+    step (seed = step * world + rank), running bpp / IoU every ``display_step``, evaluation and checkpoint every ``save_step``,
+    ``log.jsonl``.  ``make_trainer(codec, weights)`` builds the rank-local trainer, ``evaluate_fn(weights, files, device)`` scores
+    held-out cubes, ``rate_keys`` are the bpp terms it reports.  Returns the trainer."""
     import torch
     import torch.distributed as dist
-    from . import runtime, training, weights as W
+    from . import runtime, weights as W
     from .dataprocess import inout_points
 
     world = dist.get_world_size() if dist.is_initialized() else 1
@@ -191,17 +196,16 @@ def train(files: Sequence[str], ckpt_dir: str, alpha=2.0, beta=3.0, gamma=1.0, d
     # variables and the global step restarts at 0
     resume = os.path.exists(os.path.join(ckpt_dir, "weights.npz")) and load_train_state(ckpt_dir) is not None
     src = ckpt_dir if resume else init_ckpt_dir
-    w0 = W.load(src, "voxception") if src else None
-    codec = runtime.get_codec("voxception", "", device)
-    tr = training.HyperTrainer(codec, weights=w0, alpha=alpha, beta=beta, gamma=gamma, delta=delta, lr=lr, lower_bound=lower_bound,
-                               distortion=distortion)
+    w0 = W.load(src, model) if src else None
+    codec = runtime.get_codec(model, "", device)
+    tr = make_trainer(codec, w0)
     step0 = restore(tr, load_train_state(src) if src else None, with_opt)
     if not resume:
         step0 = 0
     data = CubeFiles(files, rank=rank)
     for _ in range(step0):                                            # a resumed run continues the sampling sequence
         data.sample_train(batch_size)
-    sums = {"bpp_ae": 0.0, "bpp_hyper": 0.0, "IoU": 0.0}
+    sums = {k: 0.0 for k in tuple(rate_keys) + ("IoU",)}
     num = 0
     start = time.time()
     logf = None
@@ -214,6 +218,9 @@ def train(files: Sequence[str], ckpt_dir: str, alpha=2.0, beta=3.0, gamma=1.0, d
             logf.write(json.dumps(rec) + "\n")
             logf.flush()
 
+    def bpps(d):
+        return " + ".join("%.4f" % d[k] for k in rate_keys)
+
     for step in range(step0, int(num_iteration)):
         vox = CubeFiles.voxels(data.sample_train(batch_size))
         out = tr.train_step(vox, seed=step * world + rank, group=None)
@@ -222,23 +229,25 @@ def train(files: Sequence[str], ckpt_dir: str, alpha=2.0, beta=3.0, gamma=1.0, d
             raise FloatingPointError("non-finite loss at step %d: %s" % (step, terms))
         nums = vox.reshape(len(vox), -1).sum(1).astype(np.int32)
         mask = inout_points.select_voxels(runtime.DeviceResult(out["x_tilde"]), nums, 1.0, codec=codec, dtype="uint8")
-        sums["bpp_ae"] += terms["bpp_ae"]; sums["bpp_hyper"] += terms["bpp_hyper"]; sums["IoU"] += iou(mask, vox)
+        for k in rate_keys:
+            sums[k] += terms[k]
+        sums["IoU"] += iou(mask, vox)
         num += 1
         if (step + 1) % display_step == 0:
-            rec = {"event": "train", "iteration": step, "bpp_ae": sums["bpp_ae"] / num, "bpp_hyper": sums["bpp_hyper"] / num,
-                   "IoU": sums["IoU"] / num, "loss": terms["loss"], "minutes": round((time.time() - start) / 60.0, 2)}
+            rec = {"event": "train", "iteration": step}
+            rec.update({k: sums[k] / num for k in rate_keys})
+            rec.update({"IoU": sums["IoU"] / num, "loss": terms["loss"], "minutes": round((time.time() - start) / 60.0, 2)})
             if rank == 0:
-                log("Iteration:%d\nBpps: %.4f + %.4f\nIoU: %.4f\nRunning time:(mins): %s\n" % (step, rec["bpp_ae"], rec["bpp_hyper"], rec["IoU"],
-                                                                                             rec["minutes"]))
+                log("Iteration:%d\nBpps: %s\nIoU: %.4f\nRunning time:(mins): %s\n" % (step, bpps(rec), rec["IoU"], rec["minutes"]))
                 emit(rec)
             sums = {k: 0.0 for k in sums}
             num = 0
         if (step + 1) % save_step == 0:
             if rank == 0:
                 log("evaluating...")
-                ev = evaluate(tr.export_weights(), data.sample_eval(eval_cubes), batch_size=8, device=device) if data.eval_list else {}
+                ev = evaluate_fn(tr.export_weights(), data.sample_eval(eval_cubes), device) if data.eval_list else {}
                 if ev:
-                    log("Bpps: %.4f + %.4f\nIoU: %.4f" % (ev["bpp_ae"], ev["bpp_hyper"], ev["IoU"]))
+                    log("Bpps: %s\nIoU: %.4f" % (bpps(ev), ev["IoU"]))
                     emit(dict(ev, event="eval", iteration=step))
                 save_checkpoint(ckpt_dir, tr, step + 1, with_opt)
             if world > 1:
@@ -248,12 +257,24 @@ def train(files: Sequence[str], ckpt_dir: str, alpha=2.0, beta=3.0, gamma=1.0, d
     return tr
 
 
-def main(argv=None):
-    p = argparse.ArgumentParser(formatter_class=argparse.ArgumentDefaultsHelpFormatter)
+def train(files: Sequence[str], ckpt_dir: str, alpha=2.0, beta=3.0, gamma=1.0, delta=1.0, lr=1e-5, num_iteration=int(3e5), batch_size=8,
+          init_ckpt_dir: str = "", reset_optimizer: int = 0, lower_bound: float = 1e-9, display_step: int = DISPLAY_STEP,
+          save_step: int = SAVE_STEP, eval_cubes: int = 256, log=print, distortion: str = "bce"):
+    """``train()`` of train_hyper.py:165-266.  Returns the trainer (rank-local)."""
+    from . import training
+
+    def make_trainer(codec, w0):
+        return training.HyperTrainer(codec, weights=w0, alpha=alpha, beta=beta, gamma=gamma, delta=delta, lr=lr, lower_bound=lower_bound,
+                                     distortion=distortion)
+    return run_loop(files, ckpt_dir, "voxception", make_trainer, lambda w, f, device: evaluate(w, f, batch_size=8, device=device),
+                    ("bpp_ae", "bpp_hyper"), num_iteration, batch_size, init_ckpt_dir, reset_optimizer, display_step, save_step, eval_cubes, log)
+
+
+def add_loop_arguments(p: argparse.ArgumentParser):
+    """The command-line options both training commands share."""
     p.add_argument("--data", required=True, help="glob of per-cube point files (.h5 / .npy / .npz with key 'data')")
     p.add_argument("--alpha", type=float, default=2.0, help="weight of the distortion term (BCE) in the loss")
     p.add_argument("--beta", type=float, default=3.0, help="weight of the empty-voxel part of the BCE against the occupied part")
-    p.add_argument("--gamma", type=float, default=1.0, help="weight of the hyper-latent rate (bpp of z)")
     p.add_argument("--delta", type=float, default=1.0, help="weight of the latent rate (bpp of y)")
     p.add_argument("--lr", type=float, default=1e-5)
     p.add_argument("--num_iteration", type=int, default=int(3e5))
@@ -261,16 +282,27 @@ def main(argv=None):
     p.add_argument("--prefix", type=str, default="")
     p.add_argument("--init_ckpt_dir", type=str, default="")
     p.add_argument("--reset_optimizer", type=int, default=0)
-    p.add_argument("--lower_bound", type=float, default=1e-9)
     p.add_argument("--checkpoint_dir", type=str, default="./checkpoints")
     p.add_argument("--distortion", type=str, default="bce", choices=["bce", "focal"],
                    help="occupancy loss: bce = get_bce_loss as the reference script calls it; focal = get_focal_loss (loss.py:83-93)")
-    a = p.parse_args(argv)
+
+
+def init_distributed():
+    """One process per GPU under torchrun (WORLD_SIZE > 1): bind the local GPU and join the NCCL group."""
     import torch
     import torch.distributed as dist
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
         torch.cuda.set_device(int(os.environ.get("LOCAL_RANK", "0")))
         dist.init_process_group("nccl")
+
+
+def main(argv=None):
+    p = argparse.ArgumentParser(formatter_class=argparse.ArgumentDefaultsHelpFormatter)
+    add_loop_arguments(p)
+    p.add_argument("--gamma", type=float, default=1.0, help="weight of the hyper-latent rate (bpp of z)")
+    p.add_argument("--lower_bound", type=float, default=1e-9)
+    a = p.parse_args(argv)
+    init_distributed()
     files = sorted(glob.glob(a.data))
     ckpt = os.path.join(a.checkpoint_dir, a.prefix + "hyper|a{0:.2f}b{1:.2f}".format(a.alpha, a.beta))          # train_hyper.py:269-271
     train(files, ckpt, a.alpha, a.beta, a.gamma, a.delta, a.lr, a.num_iteration, a.batch_size, a.init_ckpt_dir, a.reset_optimizer, a.lower_bound,

@@ -215,44 +215,49 @@ def _axpy(ops: _Ops, a: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
     return a.add_(b)
 
 
-class HyperTrainer:
-    """Holds the trainable variables (Keras names / layouts) as device buffers and runs training steps."""
+class _Trainer:
+    """What every training step shares: the trainable variables (Keras names / layouts) as device buffers, the layer graph of
+    the transforms, the occupancy loss, Adam, the data-parallel all-reduce and the export to the weight-file form.
 
-    def __init__(self, codec: Optional[runtime.Codec] = None, weights: Optional[Dict[str, np.ndarray]] = None, alpha=0.75, beta=3.0, gamma=1.0,
-                 delta=1.0, lr=1e-5, lower_bound=1e-9, likelihood_bound=1e-9, distortion="bce", focal_gamma=2.0, focal_alpha=0.9):
-        """``distortion``: "bce" = ``get_bce_loss`` as ``train_hyper.py:199-203`` calls it (beta * empty + full); "focal" =
-        ``get_focal_loss`` (``loss.py:83-93``, gamma 2, alpha 0.9, a SUM over the batch) on sigmoid(x_tilde) -- the reference
-        defines it but neither train script calls it; BASELINE config 5 names it, so it is selectable and D = the focal sum."""
+    ``nets`` are the top-level checkpoint keys of the transforms this model trains; ``bottlenecks`` maps the checkpoint prefix of
+    every EntropyBottleneck it trains (``estimator/``, ``estimator_y/``) to its channel count.  A bottleneck's matrices /
+    biases / factors are held concatenated in the ``pcgc_load_bottleneck`` order under ``<prefix>matrix|bais|factor``."""
+
+    def __init__(self, codec, weights, model, nets, bottlenecks, alpha, beta, delta, lr, likelihood_bound, distortion, focal_gamma,
+                 focal_alpha):
         if distortion not in ("bce", "focal"):
             raise ValueError("distortion must be 'bce' or 'focal', got %r" % (distortion,))
         self.distortion, self.focal_gamma, self.focal_alpha = distortion, float(focal_gamma), float(focal_alpha)
-        self.codec = codec or runtime.get_codec("voxception", "")
+        self.model, self.nets, self.bottlenecks = model, tuple(nets), dict(bottlenecks)
+        self.codec = codec or runtime.get_codec(model, "")
         self.ops = _Ops(self.codec)
-        w = weights if weights is not None else W.synthetic_weights("voxception")
+        w = weights if weights is not None else W.synthetic_weights(model)
         dev = self.codec.dev
         self.params: Dict[str, torch.Tensor] = {}
-        for net in _NETS:
-            for l in netspec.NETS[("voxception", net)]:
+        for net in self.nets:
+            for l in netspec.NETS[(model, net)]:
                 for kind in ("kernel", "bias"):
                     key = "%s/%s/%s" % (net, l.name, kind)
                     if key in w:
                         self.params[key] = torch.tensor(np.ascontiguousarray(w[key], dtype=np.float32), device=dev, requires_grad=True)
-        cat = lambda name: np.concatenate([np.asarray(w["estimator/%s_%d" % (name, i)], np.float32).reshape(-1) for i in range(4)])
-        for name in ("matrix", "bais", "factor"):
-            self.params["estimator/" + name] = torch.tensor(cat(name), device=dev, requires_grad=True)
-        self.alpha, self.beta, self.gamma, self.delta = float(alpha), float(beta), float(gamma), float(delta)
-        self.lr, self.lower_bound, self.likelihood_bound = float(lr), float(lower_bound), float(likelihood_bound)
+        for prefix in self.bottlenecks:
+            cat = lambda name: np.concatenate([np.asarray(w["%s%s_%d" % (prefix, name, i)], np.float32).reshape(-1) for i in range(4)])
+            for name in ("matrix", "bais", "factor"):
+                self.params[prefix + name] = torch.tensor(cat(name), device=dev, requires_grad=True)
+        self.alpha, self.beta, self.delta = float(alpha), float(beta), float(delta)
+        self.lr, self.likelihood_bound = float(lr), float(likelihood_bound)
         self.step_count = 0
         self.adam_m = {k: torch.zeros_like(v) for k, v in self.params.items()}
         self.adam_v = {k: torch.zeros_like(v) for k, v in self.params.items()}
 
-    # ---- the graph (models/model_voxception.py) ---------------------------------------------------------------------------
+    # ---- the graph (models/model_voxception.py, models/model_simple.py) ---------------------------------------------------
     def _conv(self, x, net: str, l: netspec.Layer):
         return _Conv.apply(x, self.params["%s/%s/kernel" % (net, l.name)], self.params.get("%s/%s/bias" % (net, l.name)), self.ops, l)
 
     def _run(self, net: str, x):
-        layers = {l.name: l for l in netspec.NETS[("voxception", net)]}
-        names = [l.name for l in netspec.NETS[("voxception", net)]]
+        table = netspec.NETS[(self.model, net)]
+        layers = {l.name: l for l in table}
+        names = [l.name for l in table]
         i = 0
         while i < len(names):
             n = names[i]
@@ -270,34 +275,20 @@ class HyperTrainer:
                 i += 1
         return x
 
-    def _hyper_decoder(self, z_t):
-        layers = {l.name: l for l in netspec.NETS[("voxception", "hyper_decoder")]}
-        f = self._conv(z_t, "hyper_decoder", layers["deconv1"])
-        f = self._conv(f, "hyper_decoder", layers["deconv2"])
-        f = self._conv(f, "hyper_decoder", layers["deconv3"])
-        return self._conv(f, "hyper_decoder", layers["deconv4_1"]), self._conv(f, "hyper_decoder", layers["deconv4_2"])
-
-    def forward_backward(self, cubes, seed: int = 0):
-        """cubes uint8 [B,64,64,64,1] (host or device) -> dict of loss terms (device scalars) with .grad set on every parameter."""
-        c, ops = self.codec, self.ops
+    def _begin(self, cubes):
+        """-> (label uint8, x float32, num_points) on the device; clears every gradient."""
+        c = self.codec
         label = c.to_device(cubes, torch.uint8)
         x = torch.empty(label.shape, dtype=torch.float32, device=c.dev)
         x.copy_(label)                                                    # dtype conversion of the input buffer
         num_points = int(np.count_nonzero(runtime.unwrap(cubes))) if not isinstance(cubes, torch.Tensor) else int(label.count_nonzero())
         for p in self.params.values():
             p.grad = None
-        stats: dict = {}
-        coef_y = self.delta / (-math.log(2.0) * num_points)
-        coef_z = self.gamma / (-math.log(2.0) * num_points)
-        y = self._run("analysis_transform", x)
-        z = self._run("hyper_encoder", y)
-        z_t = _FactorizedRate.apply(z, self.params["estimator/matrix"], self.params["estimator/bais"], self.params["estimator/factor"], coef_z, seed,
-                                    self.likelihood_bound, ops, stats)
-        loc, s_raw = self._hyper_decoder(z_t)
-        scale = _AbsFloor.apply(s_raw, self.lower_bound, ops)
-        y_t = _LaplaceRate.apply(y, loc, scale, coef_y, seed, self.likelihood_bound, ops, stats)
-        x_t = self._run("synthesis_transform", y_t)
-        # distortion: loss sums on the device, its gradient seeds the backward pass
+        return label, x, num_points
+
+    def _distortion_backward(self, x_t, label):
+        """Occupancy loss sums on the device; its gradient seeds the backward pass.  -> {"bce_sums" | "focal_sums": sums}."""
+        c = self.codec
         g = torch.empty_like(x_t)
         c._stream()
         if self.distortion == "focal":
@@ -311,24 +302,16 @@ class HyperTrainer:
             c._check(c.lib.pcgc_train_bce_backward(c.ctx, x_t.data_ptr(), label.data_ptr(), x_t.numel(), sums.data_ptr(), self.alpha * self.beta,
                                                    self.alpha, g.data_ptr()))
         x_t.backward(g)
-        return {"bce_sums" if self.distortion == "bce" else "focal_sums": sums, "bits_y": stats["bits_y"], "logsum_z": stats["logsum_z"],
-                "num_points": num_points, "x_tilde": x_t.detach()}
+        return {"bce_sums" if self.distortion == "bce" else "focal_sums": sums}
 
-    def loss_terms(self, out) -> Dict[str, float]:
-        """Host values of the step's loss terms (one synchronisation)."""
-        n = out["num_points"]
-        bpp_y = float(out["bits_y"].sum().item()) / n
-        bpp_z = float(out["logsum_z"].item()) / (-math.log(2.0) * n)
+    def _distortion_terms(self, out) -> Dict[str, float]:
+        """Host values of the occupancy loss: its parts and ``distortion`` (one synchronisation)."""
         if "focal_sums" in out:
             s = out["focal_sums"].cpu().numpy()
-            dist = float(s[0] + s[1])
-            return {"focal_full": float(s[0]), "focal_empty": float(s[1]), "distortion": dist, "bpp_ae": bpp_y, "bpp_hyper": bpp_z,
-                    "loss": float(self.alpha * dist + self.delta * bpp_y + self.gamma * bpp_z)}
+            return {"focal_full": float(s[0]), "focal_empty": float(s[1]), "distortion": float(s[0] + s[1])}
         s = out["bce_sums"].cpu().numpy()
         zeros, ones = s[0] / max(s[2], 1.0), s[1] / max(s[3], 1.0)
-        dist = self.beta * zeros + ones
-        return {"zeros": float(zeros), "ones": float(ones), "distortion": float(dist), "bpp_ae": bpp_y, "bpp_hyper": bpp_z,
-                "loss": float(self.alpha * dist + self.delta * bpp_y + self.gamma * bpp_z)}
+        return {"zeros": float(zeros), "ones": float(ones), "distortion": float(self.beta * zeros + ones)}
 
     def adam_step(self, beta1=0.9, beta2=0.999, eps=1e-8):
         """tf.train.AdamOptimizer.apply_gradients: lr_t = lr * sqrt(1 - beta2^t) / (1 - beta1^t); p -= lr_t * m / (sqrt(v) + eps)."""
@@ -346,7 +329,7 @@ class HyperTrainer:
 
     def allreduce_gradients(self, group=None):
         """Data-parallel training (SURVEY.md 8f rank 4): average the gradients over the ranks of a torch.distributed group
-        (NCCL over NVLink) -- ONE all-reduce of a flat ~2.6 MB buffer, then scattered back into the per-variable gradients."""
+        (NCCL over NVLink) -- ONE all-reduce of a flat buffer, then scattered back into the per-variable gradients."""
         import torch.distributed as dist
         if not dist.is_initialized() or dist.get_world_size(group) == 1:
             return
@@ -367,15 +350,108 @@ class HyperTrainer:
         return out
 
     def export_weights(self) -> Dict[str, np.ndarray]:
-        """Back to the weight-file form (Keras names; estimator variables split into matrix_i / bais_i / factor_i)."""
-        out = {k: v.detach().cpu().numpy() for k, v in self.params.items() if not k.startswith("estimator/")}
-        Cz = netspec.HYPER_CHANNELS
-        shapes = {"matrix": [(Cz, 3, 1), (Cz, 3, 3), (Cz, 3, 3), (Cz, 1, 3)], "bais": [(Cz, 3, 1)] * 3 + [(Cz, 1, 1)], "factor": [(Cz, 3, 1)] * 3 + [(Cz, 1, 1)]}
-        for name, shp in shapes.items():
-            flat = self.params["estimator/" + name].detach().cpu().numpy()
-            o = 0
-            for i, s in enumerate(shp):
-                n = int(np.prod(s))
-                out["estimator/%s_%d" % (name, i)] = flat[o:o + n].reshape(s).copy()
-                o += n
+        """Back to the weight-file form (Keras names; bottleneck variables split into <prefix>matrix_i / bais_i / factor_i)."""
+        out = {k: v.detach().cpu().numpy() for k, v in self.params.items() if not k.startswith(tuple(self.bottlenecks))}
+        for prefix, Cz in self.bottlenecks.items():
+            shapes = {"matrix": [(Cz, 3, 1), (Cz, 3, 3), (Cz, 3, 3), (Cz, 1, 3)], "bais": [(Cz, 3, 1)] * 3 + [(Cz, 1, 1)],
+                      "factor": [(Cz, 3, 1)] * 3 + [(Cz, 1, 1)]}
+            for name, shp in shapes.items():
+                flat = self.params[prefix + name].detach().cpu().numpy()
+                o = 0
+                for i, s in enumerate(shp):
+                    n = int(np.prod(s))
+                    out["%s%s_%d" % (prefix, name, i)] = flat[o:o + n].reshape(s).copy()
+                    o += n
         return out
+
+
+class HyperTrainer(_Trainer):
+    """The hyperprior model (Voxception transforms, hyper encoder / decoder, EntropyBottleneck on z, conditional model on y)."""
+
+    def __init__(self, codec: Optional[runtime.Codec] = None, weights: Optional[Dict[str, np.ndarray]] = None, alpha=0.75, beta=3.0, gamma=1.0,
+                 delta=1.0, lr=1e-5, lower_bound=1e-9, likelihood_bound=1e-9, distortion="bce", focal_gamma=2.0, focal_alpha=0.9):
+        """``distortion``: "bce" = ``get_bce_loss`` as ``train_hyper.py:199-203`` calls it (beta * empty + full); "focal" =
+        ``get_focal_loss`` (``loss.py:83-93``, gamma 2, alpha 0.9, a SUM over the batch) on sigmoid(x_tilde) -- the reference
+        defines it but neither train script calls it; BASELINE config 5 names it, so it is selectable and D = the focal sum."""
+        super().__init__(codec, weights, "voxception", _NETS, {"estimator/": netspec.HYPER_CHANNELS}, alpha, beta, delta, lr, likelihood_bound,
+                         distortion, focal_gamma, focal_alpha)
+        self.gamma, self.lower_bound = float(gamma), float(lower_bound)
+
+    def _hyper_decoder(self, z_t):
+        layers = {l.name: l for l in netspec.NETS[("voxception", "hyper_decoder")]}
+        f = self._conv(z_t, "hyper_decoder", layers["deconv1"])
+        f = self._conv(f, "hyper_decoder", layers["deconv2"])
+        f = self._conv(f, "hyper_decoder", layers["deconv3"])
+        return self._conv(f, "hyper_decoder", layers["deconv4_1"]), self._conv(f, "hyper_decoder", layers["deconv4_2"])
+
+    def forward_backward(self, cubes, seed: int = 0):
+        """cubes uint8 [B,64,64,64,1] (host or device) -> dict of loss terms (device scalars) with .grad set on every parameter."""
+        ops = self.ops
+        label, x, num_points = self._begin(cubes)
+        stats: dict = {}
+        coef_y = self.delta / (-math.log(2.0) * num_points)
+        coef_z = self.gamma / (-math.log(2.0) * num_points)
+        y = self._run("analysis_transform", x)
+        z = self._run("hyper_encoder", y)
+        z_t = _FactorizedRate.apply(z, self.params["estimator/matrix"], self.params["estimator/bais"], self.params["estimator/factor"], coef_z, seed,
+                                    self.likelihood_bound, ops, stats)
+        loc, s_raw = self._hyper_decoder(z_t)
+        scale = _AbsFloor.apply(s_raw, self.lower_bound, ops)
+        y_t = _LaplaceRate.apply(y, loc, scale, coef_y, seed, self.likelihood_bound, ops, stats)
+        x_t = self._run("synthesis_transform", y_t)
+        out = self._distortion_backward(x_t, label)
+        out.update({"bits_y": stats["bits_y"], "logsum_z": stats["logsum_z"], "num_points": num_points, "x_tilde": x_t.detach()})
+        return out
+
+    def loss_terms(self, out) -> Dict[str, float]:
+        """Host values of the step's loss terms (one synchronisation)."""
+        n = out["num_points"]
+        bpp_y = float(out["bits_y"].sum().item()) / n
+        bpp_z = float(out["logsum_z"].item()) / (-math.log(2.0) * n)
+        t = self._distortion_terms(out)
+        t.update({"bpp_ae": bpp_y, "bpp_hyper": bpp_z, "loss": float(self.alpha * t["distortion"] + self.delta * bpp_y + self.gamma * bpp_z)})
+        return t
+
+
+class FactorizedTrainer(_Trainer):
+    """The factorized-prior model: analysis -> ``EntropyBottleneck(y, training=True)`` -> synthesis, for ``model_simple`` (32-channel
+    y, the ``estimator/*`` variables) or the Voxception transforms (16-channel y, ``estimator_y/*``: the slot the codec's factorized
+    path loads; no hyper nets).
+
+    The loss is ``alpha * (beta * empty + full) + delta * bpp_y`` with the BCE (or ``alpha * focal`` with ``distortion="focal"``):
+    the hyperprior step of ``HyperTrainer`` with its hyperprior terms removed.  The reference's ``train_factorized.py`` is not
+    available, so this is this project's definition of the factorized training loss, not a parity claim.  The noise on y is the
+    factorized training stream of ``pcgc_train_factorized_forward`` seeded with the step's ``seed`` (the stream z draws from in
+    the hyperprior step)."""
+
+    def __init__(self, codec: Optional[runtime.Codec] = None, weights: Optional[Dict[str, np.ndarray]] = None, model: str = "simple", alpha=0.75,
+                 beta=3.0, delta=1.0, lr=1e-5, likelihood_bound=1e-9, distortion="bce", focal_gamma=2.0, focal_alpha=0.9):
+        if model not in ("simple", "voxception"):
+            raise ValueError("model must be 'simple' or 'voxception', got %r" % (model,))
+        prefix = "estimator/" if model == "simple" else "estimator_y/"
+        super().__init__(codec or runtime.get_codec(model, ""), weights, model, ("analysis_transform", "synthesis_transform"),
+                         {prefix: netspec.LATENT_CHANNELS[model]}, alpha, beta, delta, lr, likelihood_bound, distortion, focal_gamma, focal_alpha)
+        if self.codec.model != model:
+            raise ValueError("the codec runs model %r, the trainer %r" % (self.codec.model, model))
+        self.prefix = prefix
+
+    def forward_backward(self, cubes, seed: int = 0):
+        """cubes uint8 [B,64,64,64,1] (host or device) -> dict of loss terms (device scalars) with .grad set on every parameter."""
+        label, x, num_points = self._begin(cubes)
+        stats: dict = {}
+        coef_y = self.delta / (-math.log(2.0) * num_points)
+        y = self._run("analysis_transform", x)
+        p = self.prefix
+        y_t = _FactorizedRate.apply(y, self.params[p + "matrix"], self.params[p + "bais"], self.params[p + "factor"], coef_y, seed,
+                                    self.likelihood_bound, self.ops, stats)
+        x_t = self._run("synthesis_transform", y_t)
+        out = self._distortion_backward(x_t, label)
+        out.update({"logsum_y": stats["logsum_z"], "num_points": num_points, "x_tilde": x_t.detach()})
+        return out
+
+    def loss_terms(self, out) -> Dict[str, float]:
+        """Host values of the step's loss terms (one synchronisation)."""
+        bpp_y = float(out["logsum_y"].item()) / (-math.log(2.0) * out["num_points"])
+        t = self._distortion_terms(out)
+        t.update({"bpp_ae": bpp_y, "loss": float(self.alpha * t["distortion"] + self.delta * bpp_y)})
+        return t
