@@ -33,8 +33,7 @@ def _deps_mtime() -> float:
 # copy's bit for bit: no mul+add contraction there (the host objects are built with -ffp-contract=off).
 # metrics.cu computes the per-point D1 / D2 values in NumPy's arithmetic (every multiply and add rounded on its own); so does
 # meshsample.cu for the face weights, the sample points and their grid cells, which a NumPy restatement reproduces bit for bit.
-PER_FILE = {"entropy.cu": ["-fmad=false"] + os.environ.get("PCGC_ENTROPY_FLAGS", "").split(), "metrics.cu": ["-fmad=false"],
-            "meshsample.cu": ["-fmad=false"]}
+PER_FILE = {"entropy.cu": ["-fmad=false"], "metrics.cu": ["-fmad=false"], "meshsample.cu": ["-fmad=false"]}
 
 
 def _compile(src: str, verbose: bool) -> str:

@@ -72,17 +72,7 @@ PCGC_HD float cdf_score(float m, int v, float scale) {
   }
   return (float)((double)m * (double)scale * pcgc_ln1p_tab[v] - 1.0);
 }
-// deficits above this go through the water-filling pass first.  A pure speed knob: both routes give the step-by-step greedy's
-// counts.  On the GPU the threshold is set by the WARP, not by the row: some lane of almost every warp takes the water-filling pass
-// anyway, so what a lower threshold buys is a shorter greedy loop for the slowest lane (r02, 64 cubes of the vox10 cloud, intervals /
-// rows kernel: 2n + 8 -> 1.26 / 1.24 ms, n + 2 -> 1.15 / 1.12 ms, n/2 + 2 -> 1.16 / 1.13 ms, 4 -> 2.10 / 2.05 ms; identical bits).
-#ifndef PCGC_WATERFILL_MIN
-#define PCGC_WATERFILL_MIN(n) ((n) + 2)
-#endif
 #define PCGC_SCORE_TOL(mx) (4e-6f * fabsf(mx) + 1e-9f)
-#ifndef PCGC_CDF_ITER_HOOK
-#define PCGC_CDF_ITER_HOOK ((void)0)   // dev hook: count the greedy loop's iterations
-#endif
 
 // Largest u >= 1 with cdf_gain(m, u) >= lambda (0 if none), i.e. u <= 1 / (2^(lambda/m) - 1).  Closed form with a short
 // exact check only when the bound is within rounding distance of an integer.
@@ -128,7 +118,11 @@ PCGC_HD_NOINLINE int quantize_pmf_row(const float* pmf, int n, int precision, in
   // Every increment whose gain is >= lambda is granted at once, for a lambda that admits at most `todo` increments;
   // per-entry gains are strictly decreasing, so these are exactly the greedy's first picks.  lambda comes from the
   // continuous solution gain_i(u) ~ m_i*log2(e)/(u + 0.5), aimed a little short so that the pass is feasible.
-  for (int pass = 0; pass < 8 && dir > 0 && todo > PCGC_WATERFILL_MIN(n); ++pass) {
+  // Deficits above n + 2 take this pass, a pure speed choice: both routes give the step-by-step greedy's counts.  On the GPU the
+  // threshold is set by the WARP, not by the row: some lane of almost every warp takes the water-filling pass anyway, so what a lower
+  // threshold buys is a shorter greedy loop for the slowest lane (r02, 64 cubes of the vox10 cloud, intervals / rows kernel:
+  // 2n + 8 -> 1.26 / 1.24 ms, n + 2 -> 1.15 / 1.12 ms, n/2 + 2 -> 1.16 / 1.13 ms, 4 -> 2.10 / 2.05 ms; identical bits).
+  for (int pass = 0; pass < 8 && dir > 0 && todo > n + 2; ++pass) {
     const double L = 1.4426950408889634;
     double m_act = 0.0, t_act = (double)target;
     int n_act = n;
@@ -172,7 +166,6 @@ PCGC_HD_NOINLINE int quantize_pmf_row(const float* pmf, int n, int precision, in
   for (int i = 0; i < n; ++i)
     g[i] = dir > 0 ? cdf_score(pmf[i], v[i], scale) : (v[i] > 1 ? -cdf_score(pmf[i], v[i] - 1, scale) : -INFINITY);
   while (todo > 0) {
-    PCGC_CDF_ITER_HOOK;
     // one pass: the best score, its (first) index and the runner-up; only a runner-up within the tolerance needs the exact path
     float mx = -INFINITY, second = -INFINITY;
     int best = -1;
@@ -196,120 +189,6 @@ PCGC_HD_NOINLINE int quantize_pmf_row(const float* pmf, int n, int precision, in
     }
     v[best] += dir;
     g[best] = dir > 0 ? cdf_score(pmf[best], v[best], scale) : (v[best] > 1 ? -cdf_score(pmf[best], v[best] - 1, scale) : -INFINITY);
-    --todo;
-  }
-  return 0;
-}
-
-// ---------------------------------------------------------------------------------------------------------------------------
-// The same normaliser with its three per-row arrays in REGISTERS (r02): every loop runs over the compile-time bound NMAX with
-// an `i < n` predicate and every run-time subscript is an unrolled select, so nothing is indexed dynamically and ptxas keeps
-// pmf / v / g in registers.  The pointer form above keeps them in per-thread local memory (2 x 64 floats + 64 ints), and the CDF
-// kernels were bound by the latency of those loads (ncu r02: 38 M local loads per 64 cubes at a 10 % L1 hit rate), not by
-// instruction issue.  Operation for operation the same arithmetic in the same order as quantize_pmf_row: tools/cdf_check.cpp
-// (run by tests/test_host_coder.py) compares the host build of this template with the pointer form on ~2 M rows, and
-// tests/test_gpu_coder.py the GPU rows with the host twin's.
-// MEASURED (r02, 191 cubes of the vox10 cloud, N = 4..12): 5.57 ms against 3.36 ms for the pointer form -- the hypothesis was
-// wrong: the kernel is bound by instruction issue after all, and the NMAX-wide predicated loops and select-subscripts execute
-// about twice the instructions.  The kernels therefore use the pointer form; PCGC_CDF_REG=1 switches cubes with N <= 16 to this
-// one (kept because it is exact and shows where the time is NOT).
-template <int NMAX>
-PCGC_HD int quantize_pmf_row_reg(const float (&pmf)[NMAX], int n, int precision, int32_t (&v)[NMAX]) {
-  float g[NMAX];
-  const int target = 1 << precision;
-  const float scale = (float)target;
-  long long sum = 0;
-#pragma unroll
-  for (int i = 0; i < NMAX; ++i) {
-    int q = 0;
-    if (i < n) {
-      q = (int)rintf(pmf[i] * scale);
-      q = q < 1 ? 1 : q;
-      sum += q;
-    }
-    v[i] = q;
-    g[i] = -INFINITY;
-  }
-  long long todo = sum > target ? sum - target : target - sum;
-  if (todo == 0) return 0;
-  const int dir = sum > target ? -1 : 1;
-
-  for (int pass = 0; pass < 8 && dir > 0 && todo > PCGC_WATERFILL_MIN(n); ++pass) {
-    const double L = 1.4426950408889634;
-    double m_act = 0.0, t_act = (double)target;
-    int n_act = n;
-#pragma unroll
-    for (int i = 0; i < NMAX; ++i) if (i < n) m_act += (double)pmf[i];
-    double inv_lambda = 0.0;
-    for (int it = 0; it < 4 && m_act > 0.0; ++it) {
-      const double slack = 2.0 * sqrt((double)n_act / 12.0) + 1.0;
-      inv_lambda = (t_act - slack) / (L * m_act);
-      double t2 = (double)target, m2 = 0.0;
-      int n2 = 0;
-#pragma unroll
-      for (int i = 0; i < NMAX; ++i) if (i < n) {
-        if ((double)pmf[i] * L * inv_lambda >= (double)v[i]) { m2 += (double)pmf[i]; ++n2; } else { t2 -= (double)v[i]; }
-      }
-      if (n2 == n_act && m2 == m_act) break;
-      t_act = t2; m_act = m2; n_act = n2;
-      if (n2 == 0) break;
-    }
-    if (!(inv_lambda > 0.0) || n_act == 0) break;
-    double lambda = 1.0 / inv_lambda;
-    bool done = false;
-    for (int attempt = 0; attempt < 8 && !done; ++attempt) {
-      long long granted = 0;
-#pragma unroll
-      for (int i = 0; i < NMAX; ++i) if (i < n) {
-        long long lu = cdf_last_u((double)pmf[i], lambda);
-        if (lu > 2 * (long long)target) lu = 2 * (long long)target;
-        g[i] = (float)lu;
-        if (lu >= v[i]) granted += lu - v[i] + 1;
-      }
-      if (granted <= todo) {
-#pragma unroll
-        for (int i = 0; i < NMAX; ++i) if (i < n) { const int32_t lu = (int32_t)g[i]; if (lu >= v[i]) v[i] = lu + 1; }
-        todo -= granted;
-        done = true;
-      } else {
-        lambda *= 1.0 + ((double)(granted - todo) + 2.0 * sqrt((double)n_act) + 2.0) / (double)target;
-      }
-    }
-    if (!done) break;
-  }
-
-#pragma unroll
-  for (int i = 0; i < NMAX; ++i)
-    g[i] = i < n ? (dir > 0 ? cdf_score(pmf[i], v[i], scale) : (v[i] > 1 ? -cdf_score(pmf[i], v[i] - 1, scale) : -INFINITY)) : -INFINITY;
-  while (todo > 0) {
-    float mx = -INFINITY, second = -INFINITY;
-    int best = -1;
-#pragma unroll
-    for (int i = 0; i < NMAX; ++i) if (i < n) {
-      const float gi = g[i];
-      if (gi > mx) { second = mx; mx = gi; best = i; }
-      else if (gi > second) second = gi;
-    }
-    if (!(mx > -INFINITY)) return -2;
-    const float thr = mx - PCGC_SCORE_TOL(mx);
-    if (second >= thr) {
-      double bs = -INFINITY;
-#pragma unroll
-      for (int i = 0; i < NMAX; ++i) if (i < n) {
-        if (g[i] >= thr) {
-          const double e = dir > 0 ? cdf_gain((double)pmf[i], v[i]) : -cdf_gain((double)pmf[i], v[i] - 1);
-          if (e > bs) { bs = e; best = i; }
-        }
-      }
-    }
-    float pb = 0.0f;
-    int vb = 0;
-#pragma unroll
-    for (int i = 0; i < NMAX; ++i) if (i == best) { pb = pmf[i]; vb = v[i]; }
-    vb += dir;
-    const float gb = dir > 0 ? cdf_score(pb, vb, scale) : (vb > 1 ? -cdf_score(pb, vb - 1, scale) : -INFINITY);
-#pragma unroll
-    for (int i = 0; i < NMAX; ++i) if (i == best) { v[i] = vb; g[i] = gb; }
     --todo;
   }
   return 0;

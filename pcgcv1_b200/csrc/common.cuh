@@ -25,16 +25,13 @@ inline void prefer_shared_carveout(K kernel) {
     (void)once_;                                                              \
   } while (0)
 
-// SMs the persistent conv kernels size their grids for: the device's SM count, optionally capped (PCGC_SM_LIMIT, experiments:
-// leaving a few SMs to the one-warp-per-cube coder kernels that run beside the conv kernels on the coder streams).
+// SMs the persistent conv kernels size their grids for: the device's SM count.
 inline int conv_sm_count() {
   static const int n = [] {
     int d = 0, v = 148;
     cudaGetDevice(&d);
     cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, d);
-    const char* e = getenv("PCGC_SM_LIMIT");
-    const int lim = e ? atoi(e) : 0;
-    return lim > 0 && lim < v ? lim : v;
+    return v;
   }();
   return n;
 }

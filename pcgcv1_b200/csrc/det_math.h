@@ -123,27 +123,6 @@ PCGC_DET void det_laplace_pmf_row(int min_v, int n, float loc, float scale, floa
   }
 }
 
-// det_laplace_pmf_row into a register array: compile-time trip count, `k < n` predicate (see quantize_pmf_row_reg).
-template <int NMAX>
-PCGC_DET void det_laplace_pmf_row_reg(int min_v, int n, float loc, float scale, float bound, float (&out)[NMAX]) {
-  float s_prev = 2.0f, c_prev = 0.0f;
-#pragma unroll
-  for (int k = 0; k < NMAX; ++k) {
-    float r = 0.0f;
-    if (k < n) {
-      const float x = (float)(min_v + k);
-      const float upper = d_add(x, 0.5f), lower = d_sub(x, 0.5f);
-      const float sgn = det_signf(d_sub(d_add(upper, lower), loc));
-      const float c_lo = (sgn == s_prev) ? c_prev : det_laplace_cdf(d_add(d_mul(-sgn, d_sub(lower, loc)), loc), loc, scale);
-      const float c_up = det_laplace_cdf(d_add(d_mul(-sgn, d_sub(upper, loc)), loc), loc, scale);
-      const float p = fabsf(d_sub(c_up, c_lo));
-      r = p > bound ? p : bound;
-      s_prev = sgn; c_prev = c_up;
-    }
-    out[k] = r;
-  }
-}
-
 // ---- EntropyBottleneck (models/entropy_model.py:72-151) for filters (3,3,3) ------------------------------------------------
 // p: 44 floats per channel as packed by pcgc_load_bottleneck: softplus(matrix), bias, tanh(factor) per layer.
 PCGC_DET float det_bn_logits(float x, const float* p) {

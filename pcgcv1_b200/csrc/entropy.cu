@@ -213,26 +213,20 @@ cudaError_t launch_laplace(const float* y, const float* loc, const float* scale,
 // r02 experiment, kept as a note: moving the three per-row arrays (pmf, counts, scores) from per-thread local memory (38 M local
 // loads per 64 cubes at a 10 % L1 hit rate, ncu) into shared memory interleaved over the block ([entry][thread], 48 KiB per 128
 // threads) made the kernel SLOWER (3.78 -> 4.90 ms per 191 cubes): 16 instead of 32 resident warps hide the exp / FP64 latencies
-// of the normaliser worse than the L2 hits of the local arrays cost.
+// of the normaliser worse than the L2 hits of the local arrays cost.  Keeping them in registers instead (NMAX-wide predicated loops,
+// select subscripts, no local memory) was slower still (5.57 against 3.36 ms per 191 cubes): the kernel is bound by instruction
+// issue, and that form executes about twice the instructions.
 constexpr int CDF_THREADS = 128;
-#ifndef PCGC_PMF_SHARED
-#define PCGC_PMF_SHARED 1
-#endif
-
-#ifndef PCGC_CDF_MINBLOCKS
-#define PCGC_CDF_MINBLOCKS 12
-#endif
 template <int MODE>
-__global__ void __launch_bounds__(CDF_THREADS, PCGC_CDF_MINBLOCKS)
+__global__ void __launch_bounds__(CDF_THREADS, 12)
 laplace_cdf_kernel(const float* __restrict__ y_hat, const float* __restrict__ loc, const float* __restrict__ scale,
                    const float* __restrict__ pmf_in, int64_t E, const int32_t* __restrict__ minmax,
                    const int64_t* __restrict__ row_offset, float bound, int precision, uint32_t* __restrict__ intervals,
-                   uint16_t* __restrict__ cdf, int32_t* __restrict__ cdf32, int* __restrict__ err, int skip_upto) {
+                   uint16_t* __restrict__ cdf, int32_t* __restrict__ cdf32, int* __restrict__ err) {
   const int b = blockIdx.y;
   const int min_v = minmax[2 * b], max_v = minmax[2 * b + 1];
   const int N = max_v - min_v + 1;
   if (N < 2 || N > PCGC_MAX_SYMBOLS) { if (threadIdx.x == 0 && blockIdx.x == 0) atomicExch(err, PCGC_ERR_BAD_RANGE); return; }
-  if (N <= skip_upto) return;                    // this cube's rows are built by a register kernel (laplace_cdf_reg_kernel)
   float pmf[PCGC_MAX_SYMBOLS];
   int32_t v[PCGC_MAX_SYMBOLS];
   float g[PCGC_MAX_SYMBOLS];
@@ -242,11 +236,7 @@ laplace_cdf_kernel(const float* __restrict__ y_hat, const float* __restrict__ lo
       for (int k = 0; k < N; ++k) pmf[k] = __ldg(pmf_in + o * N + k);
     } else {
       const float l = __ldg(loc + o), s = __ldg(scale + o);
-#if PCGC_PMF_SHARED
       det_laplace_pmf_row(min_v, N, l, s, bound, pmf);         // == max(laplace_likelihood(min_v + k), bound), shared edge evaluations
-#else
-      for (int k = 0; k < N; ++k) pmf[k] = fmaxf(laplace_likelihood((float)(min_v + k), l, s), bound);
-#endif
     }
     if (quantize_pmf_row(pmf, N, precision, v, g) != 0) { atomicExch(err, PCGC_ERR_BAD_RANGE); continue; }
     if (MODE == 1) {
@@ -268,64 +258,12 @@ laplace_cdf_kernel(const float* __restrict__ y_hat, const float* __restrict__ lo
   }
 }
 
-// Register-resident form for cubes with NLO < N <= NMAX symbols (quantize_pmf_row_reg, cdf_norm.h): pmf / counts / scores live in
-// registers, no per-thread local memory.  MODE 0: uint16 rows, 1: the interval of the element's own symbol.  A block whose cube
-// belongs to another class returns at once (the symbol range is per cube, i.e. per blockIdx.y).
-template <int MODE, int NMAX, int NLO>
-__global__ void __launch_bounds__(CDF_THREADS, NMAX <= 8 ? 8 : 5)
-laplace_cdf_reg_kernel(const float* __restrict__ y_hat, const float* __restrict__ loc, const float* __restrict__ scale, int64_t E,
-                       const int32_t* __restrict__ minmax, const int64_t* __restrict__ row_offset, float bound, int precision,
-                       uint32_t* __restrict__ intervals, uint16_t* __restrict__ cdf, int* __restrict__ err) {
-  const int b = blockIdx.y;
-  const int min_v = minmax[2 * b], max_v = minmax[2 * b + 1];
-  const int N = max_v - min_v + 1;
-  if (N <= NLO || N > NMAX) return;              // N < 2 / N > PCGC_MAX_SYMBOLS are reported by the pointer-form kernel
-  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < E; e += (int64_t)gridDim.x * blockDim.x) {
-    const size_t o = (size_t)b * E + e;
-    float pmf[NMAX];
-    int32_t v[NMAX];
-    det_laplace_pmf_row_reg<NMAX>(min_v, N, __ldg(loc + o), __ldg(scale + o), bound, pmf);
-    if (quantize_pmf_row_reg<NMAX>(pmf, N, precision, v) != 0) { atomicExch(err, PCGC_ERR_BAD_RANGE); continue; }
-    if (MODE == 1) {
-      const int sym = (int)__ldg(y_hat + o) - min_v;
-      if (sym < 0 || sym >= N) { atomicExch(err, PCGC_ERR_BAD_RANGE); intervals[o] = 0; continue; }
-      uint32_t lower = 0, width = 0;
-#pragma unroll
-      for (int k = 0; k < NMAX; ++k) {
-        lower += k < sym ? (uint32_t)v[k] : 0u;
-        width = k == sym ? (uint32_t)v[k] : width;
-      }
-      intervals[o] = lower | ((width - 1) << 16);
-    } else {
-      uint16_t* row = cdf + row_offset[b] + (size_t)e * N;
-      uint32_t acc = 0;
-#pragma unroll
-      for (int k = 0; k < NMAX; ++k) {
-        if (k < N) row[k] = (uint16_t)acc;
-        acc += (uint32_t)v[k];
-      }
-    }
-  }
-}
-
-// 0 (default): everything through the pointer-form kernel; 1: cubes with N <= 16 symbols go to the register kernels (slower,
-// see cdf_norm.h: 5.57 vs 3.36 ms per 191 cubes)
-static const bool CDF_REG = [] { const char* e = getenv("PCGC_CDF_REG"); return e ? atoi(e) != 0 : false; }();
-
-static const size_t CDF_SMEM = [] { const char* e = getenv("PCGC_CDF_PAD_KB"); return (size_t)(e ? atoi(e) : 0) * 1024; }();   // occupancy experiments
-
-// PCGC_CDF_L1 (experiment): 1 = the intervals kernel (encoder side) asks for the all-L1 carveout, 2 = the rows kernel too.  The per-thread
-// arrays of the normaliser live in local memory (3 x N x 128 B per warp, 48 warps per SM: 220 KB at N = 12), which the all-shared carveout
-// of the rest of the library leaves ~28 KB of L1 for (ncu: 10 % L1 hit rate).
-static const int CDF_L1 = [] { const char* e = getenv("PCGC_CDF_L1"); return e ? atoi(e) : 0; }();
-
+// The shared carveout of the rest of the library leaves these kernels ~28 KB of L1 for their local arrays; the all-L1 carveout made
+// them faster alone but gained nothing inside the step (r02, profiles/r02_ncu_cdf_last.txt).
 template <int MODE>
 static cudaError_t cdf_prepare() {
   static const cudaError_t once = [] {
-    if ((MODE == 1 && CDF_L1 >= 1) || (MODE == 0 && CDF_L1 >= 2))
-      cudaFuncSetAttribute(laplace_cdf_kernel<MODE>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1);
-    else
-      prefer_shared_carveout(laplace_cdf_kernel<MODE>);
+    prefer_shared_carveout(laplace_cdf_kernel<MODE>);
     return cudaFuncSetAttribute(laplace_cdf_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(96 * 1024));
   }();
   return once;
@@ -342,14 +280,8 @@ cudaError_t launch_laplace_intervals(const float* y_hat, const float* loc, const
                                      int* err_flag, cudaStream_t s, int64_t* launches) {
   cudaError_t pe = cdf_prepare<1>();
   if (pe != cudaSuccess) return pe;
-  if (CDF_REG) {
-    PCGC_CARVEOUT_ONCE((laplace_cdf_reg_kernel<1, 8, 0>)); PCGC_CARVEOUT_ONCE((laplace_cdf_reg_kernel<1, 16, 8>));
-    laplace_cdf_reg_kernel<1, 8, 0><<<cdf_grid(E, B), CDF_THREADS, 0, s>>>(y_hat, loc, scale, E, minmax, nullptr, bound, precision, intervals, nullptr, err_flag);
-    laplace_cdf_reg_kernel<1, 16, 8><<<cdf_grid(E, B), CDF_THREADS, 0, s>>>(y_hat, loc, scale, E, minmax, nullptr, bound, precision, intervals, nullptr, err_flag);
-    if (launches) *launches += 2;
-  }
-  laplace_cdf_kernel<1><<<cdf_grid(E, B), CDF_THREADS, CDF_SMEM, s>>>(y_hat, loc, scale, nullptr, E, minmax, nullptr, bound, precision,
-                                                      intervals, nullptr, nullptr, err_flag, CDF_REG ? 16 : 0);
+  laplace_cdf_kernel<1><<<cdf_grid(E, B), CDF_THREADS, 0, s>>>(y_hat, loc, scale, nullptr, E, minmax, nullptr, bound, precision,
+                                                               intervals, nullptr, nullptr, err_flag);
   if (launches) ++*launches;
   return cudaGetLastError();
 }
@@ -359,14 +291,8 @@ cudaError_t launch_laplace_cdf(const float* loc, const float* scale, int B, int6
                                int* err_flag, cudaStream_t s, int64_t* launches) {
   cudaError_t pe = cdf_prepare<0>();
   if (pe != cudaSuccess) return pe;
-  if (CDF_REG) {
-    PCGC_CARVEOUT_ONCE((laplace_cdf_reg_kernel<0, 8, 0>)); PCGC_CARVEOUT_ONCE((laplace_cdf_reg_kernel<0, 16, 8>));
-    laplace_cdf_reg_kernel<0, 8, 0><<<cdf_grid(E, B), CDF_THREADS, 0, s>>>(nullptr, loc, scale, E, minmax_dev, row_offset_dev, bound, precision, nullptr, cdf, err_flag);
-    laplace_cdf_reg_kernel<0, 16, 8><<<cdf_grid(E, B), CDF_THREADS, 0, s>>>(nullptr, loc, scale, E, minmax_dev, row_offset_dev, bound, precision, nullptr, cdf, err_flag);
-    if (launches) *launches += 2;
-  }
-  laplace_cdf_kernel<0><<<cdf_grid(E, B), CDF_THREADS, CDF_SMEM, s>>>(nullptr, loc, scale, nullptr, E, minmax_dev, row_offset_dev, bound,
-                                                      precision, nullptr, cdf, nullptr, err_flag, CDF_REG ? 16 : 0);
+  laplace_cdf_kernel<0><<<cdf_grid(E, B), CDF_THREADS, 0, s>>>(nullptr, loc, scale, nullptr, E, minmax_dev, row_offset_dev, bound,
+                                                               precision, nullptr, cdf, nullptr, err_flag);
   if (launches) ++*launches;
   return cudaGetLastError();
 }
@@ -376,8 +302,8 @@ cudaError_t launch_debug_quantize_pmf(const float* pmf, int64_t rows, const int3
                                       int32_t* cdf32, int* err_flag, cudaStream_t s, int64_t* launches) {
   cudaError_t pe = cdf_prepare<2>();
   if (pe != cudaSuccess) return pe;
-  laplace_cdf_kernel<2><<<cdf_grid(rows, 1), CDF_THREADS, CDF_SMEM, s>>>(nullptr, nullptr, nullptr, pmf, rows, minmax_dev, nullptr, 0.f,
-                                                         precision, nullptr, nullptr, cdf32, err_flag, 0);
+  laplace_cdf_kernel<2><<<cdf_grid(rows, 1), CDF_THREADS, 0, s>>>(nullptr, nullptr, nullptr, pmf, rows, minmax_dev, nullptr, 0.f,
+                                                                  precision, nullptr, nullptr, cdf32, err_flag);
   if (launches) ++*launches;
   return cudaGetLastError();
 }

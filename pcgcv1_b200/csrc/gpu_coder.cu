@@ -12,7 +12,6 @@
 //           tests size*cdf[k] <= offset; a ballot gives the symbol without a division or a serial scan.  Rows stream
 //           through a double-buffered shared-memory window (cp.async), the next 16-bit word of the string is prefetched.
 #include <stdint.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "range_coder.h"
@@ -195,15 +194,13 @@ constexpr int DEC_MAXN = 64;                    // lane-parallel search: lane k 
 // Nothing inside the 32-symbol loop touches memory: the lane's CDF entries are read into registers first, the next 16-bit
 // words of the string are prefetched one per lane and handed out by shuffles.
 template <bool WIDE>
-__global__ void __launch_bounds__(256)
+__global__ void __launch_bounds__(32)
 range_decode_rows_kernel(const uint8_t* __restrict__ packed, const int64_t* __restrict__ offsets, int B, int64_t E,
                          const uint16_t* __restrict__ rows, const int64_t* __restrict__ row_offset,
                          const int32_t* __restrict__ minmax, float* __restrict__ y_hat, int* __restrict__ err, int win_elems) {
-  extern __shared__ __align__(16) uint16_t s_rows_all[];          // [cubes per block][2][win_elems], win_elems >= DEC_G * max N of the launch
+  extern __shared__ __align__(16) uint16_t s_rows[];              // [2][win_elems], win_elems >= DEC_G * max N of the launch
   const int lane = threadIdx.x;
-  const int b = blockIdx.x * blockDim.y + threadIdx.y;            // blockDim = (32, cubes per block): one warp per cube
-  if (b >= B) return;
-  uint16_t* const s_rows = s_rows_all + (size_t)threadIdx.y * 2 * win_elems;
+  const int b = blockIdx.x;
   const unsigned FULL = 0xffffffffu;
   const int min_v = minmax[2 * b], N = minmax[2 * b + 1] - min_v + 1;
   if (N < 1 || N > (WIDE ? DEC_MAXN : 32) || DEC_G * N > win_elems) { if (lane == 0) atomicExch(err, PCGC_ERR_BAD_RANGE); return; }
@@ -398,30 +395,21 @@ range_decode_rows_narrow_kernel(const uint8_t* __restrict__ packed, const int64_
 
 }  // namespace
 
-// One-warp CTAs are placed wherever a slot is free.  Measured (r02, tools/sweep_env.sh): launched with no shared-memory
+// One-warp CTAs are placed wherever a slot is free.  Measured (r02): launched with no shared-memory
 // request the 191 encoder CTAs of the vox10 cloud ran in one of two regimes, 1.7 ms or ~6-7 ms per launch, depending on what
 // the device was finishing when the launch became runnable: the hardware scheduler stacks up to 32 such CTAs on the SMs that
 // are free at that moment and they stay there for the whole launch, so a latency-bound warp shares its scheduler with 7
 // others.  Unused dynamic shared memory per CTA caps the CTAs per SM (about B / 148 + 1, at least 2) and so forces a launch
 // to spread over the device: 1.7 ms every time.  Large launches (thousands of cubes) keep up to 32 CTAs per SM: there the
-// throughput of the SM counts, not the latency of one string.  PCGC_ENC_PAD_KB / PCGC_DEC_PAD_KB override (0 = off).
-static size_t coder_pad_bytes(const char* env, const void* kernel, int B, bool on_by_default) {
+// throughput of the SM counts, not the latency of one string.  The decoder gets no padding: its slowdown beside the synthesis is
+// issue-slot contention with the conv CTAs of the same SM, which spreading it does not change (DESIGN.md §4.3).
+static size_t encoder_pad_bytes(int B) {
   static const int max_kb = 200;
-  const char* e = getenv(env);
-  int kb;
-  if (e) {
-    kb = atoi(e);
-  } else if (on_by_default) {
-    int per_sm = (B + 147) / 148 + 1;
-    if (per_sm < 2) per_sm = 2;
-    kb = per_sm >= 32 ? 0 : max_kb / per_sm - 2;
-  } else {
-    kb = 0;
-  }
-  if (kb <= 0) return 0;
-  if (kb > max_kb - 16) kb = max_kb - 16;
-  cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_kb * 1024);
-  return (size_t)kb * 1024;
+  int per_sm = (B + 147) / 148 + 1;
+  if (per_sm < 2) per_sm = 2;
+  if (per_sm >= 32) return 0;
+  cudaFuncSetAttribute(range_encode_intervals_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_kb * 1024);
+  return (size_t)(max_kb / per_sm - 2) * 1024;
 }
 
 cudaError_t launch_range_encode_intervals(const uint32_t* iv, int B, int64_t E, int precision, uint8_t* scratch, int64_t stride,
@@ -433,8 +421,7 @@ cudaError_t launch_range_encode_intervals(const uint32_t* iv, int B, int64_t E, 
   if (precision != 16 || E % 32 || E > 65536 || stride < dig_off + 4 * (E + 2) || (stride & 15)) return cudaErrorInvalidValue;
   PCGC_CARVEOUT_ONCE(range_encode_intervals_kernel);
   PCGC_CARVEOUT_ONCE(pack_strings_kernel);
-  const size_t enc_pad = coder_pad_bytes("PCGC_ENC_PAD_KB", (const void*)range_encode_intervals_kernel, B, true);
-  range_encode_intervals_kernel<<<B, 32, enc_pad, s>>>(iv, B, E, scratch, stride, dig_off, lens);
+  range_encode_intervals_kernel<<<B, 32, encoder_pad_bytes(B), s>>>(iv, B, E, scratch, stride, dig_off, lens);
   pack_strings_kernel<<<B, 256, 0, s>>>(scratch, stride, lens, B, packed, cap, offsets, err);
   if (launches) *launches += 2;
   return cudaGetLastError();
@@ -445,27 +432,23 @@ cudaError_t launch_range_decode_rows(const uint8_t* packed, const int64_t* offse
                                      cudaStream_t s, int64_t* launches) {
   if (B <= 0) return cudaSuccess;
   if (E % DEC_G || max_n < 1 || max_n > DEC_MAXN || precision != 16) return cudaErrorInvalidValue;
-  if (max_n <= 31 && (reinterpret_cast<uintptr_t>(rows) & 15) == 0 && !getenv("PCGC_DEC_WIDE")) {
+  if (max_n <= 31 && (reinterpret_cast<uintptr_t>(rows) & 15) == 0) {
     // every row window is a multiple of 64 bytes (E % 32 == 0), so 16-byte cp.async needs only the base pointer aligned
     const int slot_elems = (32 * max_n + 32 + 7) / 8 * 8;
     PCGC_CARVEOUT_ONCE(range_decode_rows_narrow_kernel);
-    const size_t dec_pad = coder_pad_bytes("PCGC_DEC_PAD_KB", (const void*)range_decode_rows_narrow_kernel, B, false);
-    range_decode_rows_narrow_kernel<<<B, 32, (size_t)DECN_SLOTS * slot_elems * sizeof(uint16_t) + dec_pad, s>>>(packed, offsets, B, E, rows, row_offset, minmax,
-                                                                                                    y_hat, err, slot_elems);
+    range_decode_rows_narrow_kernel<<<B, 32, (size_t)DECN_SLOTS * slot_elems * sizeof(uint16_t), s>>>(packed, offsets, B, E, rows, row_offset,
+                                                                                                      minmax, y_hat, err, slot_elems);
     if (launches) ++*launches;
     return cudaGetLastError();
   }
   const int win_elems = DEC_G * ((max_n + 7) / 8 * 8);              // 16-byte multiple per window
-  // cubes (= warps) per block.  1 spreads the decoder warps over all SMs; more packs them onto few SMs (experiments: PCGC_DEC_CPB)
-  static const int cpb = [] { const char* e = getenv("PCGC_DEC_CPB"); const int v = e ? atoi(e) : 1; return v < 1 ? 1 : (v > 8 ? 8 : v); }();
-  const size_t smem = (size_t)cpb * 2 * win_elems * sizeof(uint16_t);
+  const size_t smem = 2 * (size_t)win_elems * sizeof(uint16_t);
   PCGC_CARVEOUT_ONCE(range_decode_rows_kernel<true>);
   PCGC_CARVEOUT_ONCE(range_decode_rows_kernel<false>);
-  const dim3 block(32, cpb), grid((B + cpb - 1) / cpb);
   if (max_n > 32)
-    range_decode_rows_kernel<true><<<grid, block, smem, s>>>(packed, offsets, B, E, rows, row_offset, minmax, y_hat, err, win_elems);
+    range_decode_rows_kernel<true><<<B, 32, smem, s>>>(packed, offsets, B, E, rows, row_offset, minmax, y_hat, err, win_elems);
   else
-    range_decode_rows_kernel<false><<<grid, block, smem, s>>>(packed, offsets, B, E, rows, row_offset, minmax, y_hat, err, win_elems);
+    range_decode_rows_kernel<false><<<B, 32, smem, s>>>(packed, offsets, B, E, rows, row_offset, minmax, y_hat, err, win_elems);
   if (launches) ++*launches;
   return cudaGetLastError();
 }

@@ -114,26 +114,23 @@ def decompress_factorized(strings, min_v, max_v, shape, model, ckpt_dir):
 # The batch is processed in chunks as a two-stage software pipeline: while the host range coder (worker thread; the C
 # entry points release the GIL and fan out over their own thread pool) works on chunk k, the GPU already runs the
 # transforms of chunk k+1 and a copy stream moves the coder's inputs through rotating pinned buffers.
-_CHUNK = int(os.environ.get("PCGC_CHUNK", "64"))
-_CHUNK_EDGE = int(os.environ.get("PCGC_CHUNK_EDGE", "16"))
-_CHUNK_RAMP = bool(int(os.environ.get("PCGC_CHUNK_RAMP", "1")))
+_CHUNK = 64
+_CHUNK_EDGE = 16
 _FACT_PART = int(os.environ.get("PCGC_FACT_PART", "48"))      # cubes per synthesis call of the progressive factorized decoder
-_ROWS_ON_MAIN = bool(int(os.environ.get("PCGC_ROWS_ON_MAIN", "0")))   # measured r02: 32.1 ms (rows on main) vs 31.6 ms (rows beside the conv kernels)
-_Z_EARLY = bool(int(os.environ.get("PCGC_Z_EARLY", "1")))     # hyper string coded from the staged copy of z while the GPU finishes
 
 
 def _chunks(B, small_first=False, small_last=False):
     """[a, b) chunk bounds.  The pipeline's exposed latency is one chunk's host-coder round trip at the start of a decode
     (nothing can be synthesised before the first chunk is decoded) and at the end of an encode (the last chunk's strings):
-    those chunks are small (PCGC_CHUNK_EDGE cubes), the ones in between large (PCGC_CHUNK)."""
-    e = _CHUNK_EDGE if 0 < _CHUNK_EDGE < _CHUNK else 0
+    those chunks are small (_CHUNK_EDGE cubes), the ones in between large (_CHUNK)."""
+    e = _CHUNK_EDGE
     lo, hi = 0, B
     head, tail = [], []
-    if small_first and e and B > 2 * e:
+    if small_first and B > 2 * e:
         head.append((0, e)); lo = e
-        if _CHUNK_RAMP and 2 * e < _CHUNK and hi - lo > 2 * e + _CHUNK:      # e, 2e, then full chunks: the GPU gets work early
+        if hi - lo > 2 * e + _CHUNK:                                    # e, 2e, then full chunks: the GPU gets work early
             head.append((lo, lo + 2 * e)); lo += 2 * e
-    if small_last and e and hi - lo > 2 * e:
+    if small_last and hi - lo > 2 * e:
         tail.append((hi - e, hi)); hi -= e
     mid = [(a, min(hi, a + _CHUNK)) for a in range(lo, hi, _CHUNK)]
     return head + mid + tail
@@ -143,7 +140,7 @@ def _gpu_decode_chunks(B):
     string (a few ms) whatever the number of cubes -- so the schedule starts small and grows: 8, 24, 64 cubes, then the rest
     (decoded behind the synthesis of the chunk before; a chunk's CDF rows take ~2.5 MB per cube of device memory).  Measured on
     the vox10 cloud (tools/sweep_dec.py, decompress + select): 34.2 ms with one 64-cube head, 31.3 ms with this ramp."""
-    ramp = [int(v) for v in os.environ.get("PCGC_DEC_RAMP", os.environ.get("PCGC_DEC_FIRST", "8,24,64")).split(",") if v]
+    ramp = [int(v) for v in os.environ.get("PCGC_DEC_RAMP", "8,24,64").split(",") if v]
     rest = int(os.environ.get("PCGC_DEC_CHUNK", "512"))
     if B <= max(ramp[0], 64):
         return [(0, B)]
@@ -177,21 +174,12 @@ def _pool_z():
     return _POOL_Z
 
 
-def _host_tail(B):
-    """(Opt-in, PCGC_HOST_TAIL=n; default 0.)  Cubes at the END of a compress call whose strings the host coder writes.  The GPU encoder's latency is one cube's string
-    (~4 ms, more beside the conv kernels) however few cubes it codes, so the cubes whose intervals only appear in the last few
-    milliseconds go to the host thread pool instead (0.35 ms per cube and thread); everything before them is coded on the GPU
-    while their transforms run.  Both coders write the same bytes (tests/test_gpu_coder.py)."""
-    t = int(os.environ.get("PCGC_HOST_TAIL", "0"))    # measured r02 (B200 + 16 host cores, 191 cubes): 48 -> compress 31.7 ms, 24 -> 32.5 ms,
-    return max(0, min(t, B - 1)) if B > 64 else 0      # 0 -> 28.0 ms: the worker threads' GIL traffic delays the kernel enqueue more than the tail saves
-
-
-def encode_on_device(codec, entropy_bottleneck, cem, cubes, keep_side_info=False, want_likelihoods=False, host_tail=0, z_to_host=None):
+def encode_on_device(codec, entropy_bottleneck, cem, cubes, keep_side_info=False, want_likelihoods=False, z_to_host=None):
     """Every GPU kernel of the hyper encoder for ``cubes`` (host or device resident), enqueued without a host
-    synchronisation: transforms chunk by chunk on the current stream, then ONE range-encoder launch for the first
-    B - host_tail cubes on the coder stream; the intervals of the last ``host_tail`` cubes go to pinned memory for the host
-    coder.  -> (intervals [B,E], minmax [B,2], [z_hat per chunk], [(loc, scale) per chunk], packed bytes, offsets [Bg+1],
-    [(a, b, pinned intervals, copy-done event) per tail chunk]); tensors on the device.  The caller owns the synchronisation.
+    synchronisation: transforms chunk by chunk on the current stream, then ONE range-encoder launch for all B cubes on the
+    coder stream.  -> (intervals [B,E], minmax [B,2], [z_hat per chunk], [(loc, scale) per chunk], packed bytes, offsets [B+1],
+    []); tensors on the device.  The last element is always an empty list: the 7-tuple is kept for the callers that unpack it.
+    The caller owns the synchronisation.
     ``z_to_host`` (a dict to fill): every chunk's quantised hyper latents and their (min, max) are also copied to pinned memory
     on the copy stream as soon as they exist -- ["z"] float32 [B,8,8,8,8], ["mm"] int32 [chunks,2], ["done"] an event that fires
     when the LAST chunk's copy has landed, i.e. before that chunk's hyper decoder, intervals and the range encoder have run:
@@ -202,15 +190,8 @@ def encode_on_device(codec, entropy_bottleneck, cem, cubes, keep_side_info=False
     main, side = torch.cuda.current_stream(dev), codec.coder_stream()
     iv_all = torch.empty((B, E), dtype=torch.int32, device=dev)
     mm_all = torch.empty((B, 2), dtype=torch.int32, device=dev)
-    z_hats, keep, tails = [], [], []
-    Bg = B - host_tail                                                 # cubes [0, Bg) -> GPU coder, [Bg, B) -> host coder
-    chunks = _chunks(Bg)
-    if host_tail:
-        edge = max(8, min(16, host_tail // 2))                         # the very last chunk is small: its host coding is exposed
-        mid = host_tail - edge
-        if mid > 0:
-            chunks.append((Bg, Bg + mid))
-        chunks.append((Bg + mid, B))
+    z_hats, keep = [], []
+    chunks = _chunks(B)
     # host-resident input: every chunk's H2D copy is issued up front on the copy stream, so only the first one is exposed
     uploads = None
     if not (isinstance(cubes, torch.Tensor) and cubes.is_cuda):
@@ -222,7 +203,6 @@ def encode_on_device(codec, entropy_bottleneck, cem, cubes, keep_side_info=False
                 ev = torch.cuda.Event()
                 ev.record(cs)
                 uploads.append((xc, ev))
-    packed = offsets = None
     if z_to_host is not None:
         zcs = runtime.copy_stream(dev)
         nz = B * 8 * 8 * 8 * 8
@@ -230,17 +210,7 @@ def encode_on_device(codec, entropy_bottleneck, cem, cubes, keep_side_info=False
         z_to_host["mm"] = runtime.pinned_buffer("z_mm_enc", 8 * len(chunks))[:8 * len(chunks)].view(torch.int32).view(len(chunks), 2)
         runtime.COUNTERS["d2h_bytes"] += 4 * nz + 8 * len(chunks)
 
-    def launch_gpu_coder():
-        ready = torch.cuda.Event()
-        ready.record(main)
-        iv_all.record_stream(side)
-        with torch.cuda.stream(side):
-            side.wait_event(ready)
-            return cem.encode_dev(iv_all[:Bg])
-
     for k, (a, b) in enumerate(chunks):
-        if a == Bg and packed is None and Bg > 0:
-            packed, offsets = launch_gpu_coder()                       # beside the transforms of the tail chunks
         if uploads is not None:
             x, ev = uploads[k]
             main.wait_event(ev)
@@ -265,34 +235,33 @@ def encode_on_device(codec, entropy_bottleneck, cem, cubes, keep_side_info=False
         locs, scales = codec.hyper_decode(z_hat, 1e-9)                  # lower_bound = 1e-9, transform.py:145-146
         _, mm = cem.intervals_dev(ys, locs, scales, iv_out=iv_all[a:b], want_likelihoods=want_likelihoods)
         mm_all[a:b].copy_(mm)
-        if a >= Bg:
-            stage, done = runtime.to_host_async(iv_all[a:b], "intervals%d" % (len(tails) % 2))
-            tails.append((a, b, stage, done))
         if keep_side_info:
             keep.append((locs, scales))
-    if packed is None and Bg > 0:
-        packed, offsets = launch_gpu_coder()
+    packed = offsets = None
+    if B > 0:
+        ready = torch.cuda.Event()
+        ready.record(main)
+        iv_all.record_stream(side)
+        with torch.cuda.stream(side):
+            side.wait_event(ready)
+            packed, offsets = cem.encode_dev(iv_all)
     mm_all.record_stream(side)
-    return iv_all, mm_all, z_hats, keep, packed, offsets, tails
+    return iv_all, mm_all, z_hats, keep, packed, offsets, []
 
 
 def _compress_hyper_gpu_coder(codec, entropy_bottleneck, cem, cubes, decompress, code_z=True, strings_on_device=False):
     """compress_hyper with the per-cube strings written ON THE GPU (csrc/gpu_coder.cu).  The chunks only enqueue kernels (no
     host synchronisation in the loop); the intervals land in one device buffer, ONE encoder launch codes the strings of all
-    cubes but the last few (``_host_tail``) on the coder stream, and this thread range-codes the single hyper string z on the
-    host meanwhile."""
+    cubes on the coder stream, and this thread range-codes the single hyper string z on the host meanwhile (``code_z=False``:
+    no hyper string)."""
     B = cubes.shape[0]
     side = codec.coder_stream()
-    tail = 0 if strings_on_device else _host_tail(B)
-    Bg = B - tail
     codec.deferred_checks(True)
     try:
-        z_host = {} if code_z and _Z_EARLY else None
-        iv_all, mm_all, z_hats, keep, packed, offsets, tails = encode_on_device(codec, entropy_bottleneck, cem, cubes, decompress,
-                                                                               host_tail=tail, z_to_host=z_host)
-        tail_jobs = [_pool().submit(cem.encode_finish, stage, done) for (_, _, stage, done) in tails]
-        hdr = runtime.pinned_buffer("enc_hdr", 8 * (Bg + 1))
-        off_h = hdr[:8 * (Bg + 1)].view(torch.int64)
+        z_host = {} if code_z else None
+        _, mm_all, z_hats, keep, packed, offsets, _ = encode_on_device(codec, entropy_bottleneck, cem, cubes, decompress, z_to_host=z_host)
+        hdr = runtime.pinned_buffer("enc_hdr", 8 * (B + 1))
+        off_h = hdr[:8 * (B + 1)].view(torch.int64)
         with torch.cuda.stream(side):
             off_h.copy_(offsets, non_blocking=True)
             hdr_done = torch.cuda.Event()
@@ -302,21 +271,17 @@ def _compress_hyper_gpu_coder(codec, entropy_bottleneck, cem, cubes, decompress,
         z_all = torch.cat(z_hats) if len(z_hats) > 1 else z_hats[0]
         z_string = z_min = z_max = None
         _tr("enqueued")
-        if code_z and z_host is not None:
+        if code_z:
             z_host["done"].synchronize()
             _tr("z on host")
             z_string, z_min, z_max = entropy_bottleneck.compress_quantized_host(z_host["z"].numpy(), z_host["mm"].numpy())
             _tr("z coded")
-        elif code_z:
-            sym, cdf, z_min, z_max = entropy_bottleneck.compress_begin(z_all)
-            z_string = entropy_bottleneck.compress_finish(sym, cdf)
-            _tr("z coded (late)")
         mm = runtime.to_host(mm_all).copy()
         _tr("minmax on host")
         hdr_done.synchronize()
         _tr("encoder done")
         off = off_h.numpy().copy()
-        total = int(off[Bg])
+        total = int(off[B])
         if strings_on_device:
             # sharded form: the strings stay packed in HBM (string i = packed[off[i]:off[i+1]]) and travel GPU -> GPU
             side.synchronize()
@@ -330,10 +295,8 @@ def _compress_hyper_gpu_coder(codec, entropy_bottleneck, cem, cubes, decompress,
         _tr("strings on host")
         runtime.COUNTERS["d2h_bytes"] += total + hdr.numel()
         blob = stage.numpy()
-        strings = [blob[off[i]:off[i + 1]].tobytes() for i in range(Bg)]
+        strings = [blob[off[i]:off[i + 1]].tobytes() for i in range(B)]
         _tr("strings sliced")
-        for j in tail_jobs:
-            strings += j.result()
     finally:
         codec.deferred_checks(False)
     codec.synchronize()                                                   # raises if any kernel of the section flagged an error
@@ -458,17 +421,15 @@ def _decompress_hyper_gpu_coder(codec, cem, strings, mins, maxs, y_shape, z_get,
             else:
                 packed, offs = codec.upload_strings(strings[a:b], slot=k % 4)     # this chunk's strings only: nothing waits for the rest
             locs, scales = codec.hyper_decode(z_get(a, b), 1e-9)
-            # PCGC_ROWS_ON_MAIN=1 (experiment): the CDF rows kernel on the main stream right behind the hyper decoder, only the
-            # range decoder on the side stream.  Not faster: the rows kernel then delays the synthesis of the chunk before.
-            rows_pack = cem.decode_rows_dev(locs, scales, mins[a:b], maxs[a:b]) if _ROWS_ON_MAIN else None
             ready = torch.cuda.Event()
             ready.record(main)
-            for t in (locs, scales, packed, offs) + (tuple(x for x in rows_pack if isinstance(x, torch.Tensor)) if rows_pack else ()):
+            for t in (locs, scales, packed, offs):
                 t.record_stream(side)
             with torch.cuda.stream(side):
                 side.wait_event(ready)
-                if rows_pack is None:
-                    rows_pack = cem.decode_rows_dev(locs, scales, mins[a:b], maxs[a:b])
+                # the CDF rows are built here beside the synthesis of the chunk before (r02: on the main stream they delayed
+                # that synthesis, 32.1 against 31.6 ms)
+                rows_pack = cem.decode_rows_dev(locs, scales, mins[a:b], maxs[a:b])
                 y_hat = cem.decode_strings_dev(packed, offs, rows_pack)
                 done = torch.cuda.Event()
                 done.record(side)

@@ -160,14 +160,15 @@ def test_gpu_coder_empty_and_ragged_strings(codec):
 
 
 def test_hyper_streams_do_not_depend_on_where_the_coder_runs(codec, monkeypatch):
-    """transform.compress_hyper with PCGC_CODER=gpu and =host writes the same bytes; each side decodes the other's."""
+    """transform.compress_hyper with PCGC_CODER=gpu and =host writes the same bytes (y strings and their min / max, the z string
+    and its min / max); each side decodes the other's."""
     cubes, _, nums = synthetic.workload("vox10", seed=0, max_cubes=20)
     outs = {}
     for mode in ("gpu", "host"):
         monkeypatch.setenv("PCGC_CODER", mode)
         outs[mode] = [o.numpy() for o in transform.compress_hyper(cubes, model_voxception, "")]
     g, h = outs["gpu"], outs["host"]
-    assert list(g[0]) == list(h[0]) and g[4] == h[4]
+    assert list(g[0]) == list(h[0]) and g[4] == h[4] and int(g[5]) == int(h[5]) and int(g[6]) == int(h[6])
     assert np.array_equal(g[1], h[1]) and np.array_equal(g[2], h[2])
     monkeypatch.setenv("PCGC_CODER", "gpu")
     x_gpu = transform.decompress_hyper(*h, model_voxception, "").numpy()
