@@ -217,12 +217,18 @@ struct pcgc_ctx {
   int64_t* chunk_dev = nullptr; size_t chunk_cap = 0;   // voxelize / extract workspace
   GeoWorkspace* geo_ws = nullptr;   // pcgc_geometry_sums (metrics.cu)
   MeshWorkspace* mesh_ws = nullptr; // pcgc_mesh_sample (meshsample.cu)
-  // far-field tiles of the analysis transform (PCGC_FARFIELD; DESIGN 4.1): the three VRN-16 block outputs of the all-zero cube, the
-  // classification masks of the current sub-batch
+  // far-field tiles of the analysis transform (PCGC_FARFIELD; DESIGN 4.1).  The 64^3 stage keeps each layer in a buffer of its own,
+  // ff_act = X0, T1a, X1, T1b, X2, T1c (one cube per sub-batch slot), so that a slot still holds a known layer between calls: every voxel
+  // holds the value the slot's last cube gives, which is the empty cube's value wherever that cube's tile is far.
   uint8_t* ff_zero = nullptr; float* ff_y = nullptr;
-  __nv_bfloat16* ff_e[3] = {nullptr, nullptr, nullptr};
-  uint8_t* ff_rows = nullptr; uint8_t* ff_masks = nullptr; int ff_cap = 0;
+  __nv_bfloat16* ff_e[3] = {nullptr, nullptr, nullptr};          // the empty cube's X1, X2, X3: what K_b16 copies into far tiles
+  float* ff_act[6] = {nullptr}; size_t ff_act_cap[6] = {0};
+  // classification masks [layer][ff_cap slots][128 tiles]: ff_masks of the current sub-batch (7 layers), ff_prev of the cube each slot
+  // held before (X0 .. T1c; all ones where the slot's contents are unknown)
+  uint8_t* ff_rows = nullptr; uint8_t* ff_masks = nullptr; uint8_t* ff_prev = nullptr; int ff_cap = 0;
+  int* ff_lists = nullptr;         // the work lists of K_a16 (T1a, T1b, T1c) and K_b16 (X1, X2): [5][ff_cap*1024 + 1] (launch_ff_list)
   bool ff_ready = false, ff_building = false;
+  bool ff_known = false;           // ff_prev describes the slots (cleared by anything that writes them without masks)
   int sub_batch = 64;     // cubes per kernel launch (measured r01: 64 beats 32 by 5 % with the persistent kernels; 96 and 128 add nothing)
   // optional per-launch CUDA-event timing (bench.py roofline): see pcgc_profile_enable
   bool profiling = false;
@@ -486,9 +492,10 @@ int run_vox_umma(pcgc_ctx* ctx, int kind, const float* in_ext, const void* cubes
   UmmaProgram& up = n.up;
   auto pm = [&](int buf, int nn, int c, int nb) { PmTensor t; t.p = (__nv_bfloat16*)ctx->bufs[buf]; t.n = nn; t.c = c; t.B = nb; return t; };
   auto umma = [&](const char* what, const UmmaWeights& w, const PmTensor& in, int epi, int flags, const PmTensor& out, const PmTensor& res,
-                  float* of32, int ocs, int s2d = 0, const uint8_t* ff_mask = nullptr, const __nv_bfloat16* ff_src = nullptr) -> int {
+                  float* of32, int ocs, int s2d = 0, const uint8_t* ff_mask = nullptr, const uint8_t* ff_prev = nullptr,
+                  const __nv_bfloat16* ff_src = nullptr, const int* ff_list = nullptr, int ff_list_zs = 0) -> int {
     UmmaCall c; c.out_s2d = s2d; c.in = in; c.epi = epi; c.flags = flags; c.out = out; c.res = res; c.out_f32 = of32; c.out_cs = ocs; c.out_co = 0;
-    c.err = ctx->err_flag; c.ff_mask = ff_mask; c.ff_src = ff_src;
+    c.err = ctx->err_flag; c.ff_mask = ff_mask; c.ff_prev = ff_prev; c.ff_src = ff_src; c.ff_list = ff_list; c.ff_list_zs = ff_list_zs;
     char tag[96];
     snprintf(tag, sizeof tag, "conv_umma %s c%d->%d n%d", what, w.cin, w.n_real, in.n);
     // algorithmic MACs of the reference layers this kernel stands for
@@ -530,22 +537,34 @@ int run_vox_umma(pcgc_ctx* ctx, int kind, const float* in_ext, const void* cubes
     return PCGC_OK;
   };
   const PmTensor none;
-  // Far-field tiles (analysis, uint8 cubes): a tile of a VRN-16 block whose receptive field (3 / 5 / 7 voxels for the three blocks) holds
-  // no occupied voxel equals the all-zero cube's output at the same position -- SAME padding included -- so the tile kernel copies it
-  // from the cached activations of the empty cube instead of computing it (bit-identical; 67-82 % of the tiles of the vox10 cloud).
+  // The analysis 64^3 stage writes its layers into ff_act.  Far-field tiles (uint8 cubes): a tile of layer L whose receptive field (radius
+  // L + 1: 1 for X0 .. 7 for X3) holds no occupied voxel equals the all-zero cube's value at the same position -- SAME padding included.
+  // Per slot and layer: near tiles are computed; far tiles that the slot's previous cube left near are restored (K_b16 copies them from
+  // the cached layer of the empty cube, conv_in and K_a16 compute them); the other far tiles already hold the empty cube's values and are
+  // not touched.  Bit-identical to computing every tile (67-82 % of the tiles of the vox10 cloud are far).
+  const int ff_ch[6] = {16, 8, 16, 8, 16, 8};
+  if (ana)
+    for (int L = 0; L < 6; ++L) {
+      const size_t e = (size_t)ff_ch[L] * 64 * 64 * 64 * SB;      // PM: 4 bytes per channel and voxel
+      if (ctx->ff_act_cap[L] < e) { ctx->ff_known = false; r = ensure(ctx, &ctx->ff_act[L], &ctx->ff_act_cap[L], e); if (r) return r; }
+    }
   const char* ff_env = getenv("PCGC_FARFIELD");
   const bool ff = ana && cubes_dtype == PCGC_DTYPE_U8 && !ctx->ff_building && (ff_env ? atoi(ff_env) != 0 : PCGC_FARFIELD_DEFAULT);
+  if (ana && !ff) ctx->ff_known = false;                          // every tile computed: the slots hold cubes no mask describes
   const size_t ff_cube_bytes = (size_t)4 * 64 * 64 * 64 * 8 * sizeof(__nv_bfloat16);      // one cube of a 16-channel PM tensor
   if (ff) {
     if (!ctx->ff_zero) { CK(cudaMalloc((void**)&ctx->ff_zero, 64 * 64 * 64)); CK(cudaMemsetAsync(ctx->ff_zero, 0, 64 * 64 * 64, ctx->stream)); }
     if (!ctx->ff_y) CK(cudaMalloc((void**)&ctx->ff_y, (size_t)16 * 16 * 16 * 16 * sizeof(float)));
     for (auto& e : ctx->ff_e) if (!e) CK(cudaMalloc((void**)&e, ff_cube_bytes));
     if (ctx->ff_cap < SB) {
-      if (ctx->ff_rows) cudaFree(ctx->ff_rows);
-      if (ctx->ff_masks) cudaFree(ctx->ff_masks);
-      ctx->ff_rows = ctx->ff_masks = nullptr; ctx->ff_cap = 0;
-      CK(cudaMalloc((void**)&ctx->ff_rows, (size_t)3 * SB * 4096));
-      CK(cudaMalloc((void**)&ctx->ff_masks, (size_t)3 * SB * 128));
+      CK(cudaStreamSynchronize(ctx->stream));
+      for (uint8_t** p : {&ctx->ff_rows, &ctx->ff_masks, &ctx->ff_prev}) if (*p) { cudaFree(*p); *p = nullptr; }
+      if (ctx->ff_lists) { cudaFree(ctx->ff_lists); ctx->ff_lists = nullptr; }
+      ctx->ff_cap = 0; ctx->ff_known = false;
+      CK(cudaMalloc((void**)&ctx->ff_rows, (size_t)FF_LAYERS * SB * 4096));
+      CK(cudaMalloc((void**)&ctx->ff_masks, (size_t)FF_LAYERS * SB * 128));
+      CK(cudaMalloc((void**)&ctx->ff_prev, (size_t)6 * SB * 128));
+      CK(cudaMalloc((void**)&ctx->ff_lists, (size_t)5 * ((size_t)SB * 1024 + 1) * sizeof(int)));
       ctx->ff_cap = SB;
     }
     if (!ctx->ff_ready) {                              // one pass of the empty cube with every tile computed; its block outputs are kept
@@ -555,27 +574,43 @@ int run_vox_umma(pcgc_ctx* ctx, int kind, const float* in_ext, const void* cubes
       if (rb) return rb;
       ctx->ff_ready = true;
     }
+    if (!ctx->ff_known) {                              // unknown contents: every far tile of every slot is restored once
+      CK(cudaMemsetAsync(ctx->ff_prev, 0xFF, (size_t)6 * ctx->ff_cap * 128, ctx->stream));
+      ctx->ff_known = true;
+    }
   }
+  const size_t ff_ls = (size_t)ctx->ff_cap * 128;                // mask bytes per layer
+  auto ff_cur = [&](int L) -> const uint8_t* { return ff ? ctx->ff_masks + L * ff_ls : nullptr; };
+  auto ff_old = [&](int L) -> const uint8_t* { return ff && L < 6 ? ctx->ff_prev + L * ff_ls : nullptr; };
+  // work list j: K_a16 of block i at j = 2i, K_b16 of blocks 1 and 2 at j = 1, 3
+  auto ff_list = [&](int j) -> int* { return ff ? ctx->ff_lists + (size_t)j * ((size_t)ctx->ff_cap * 1024 + 1) : nullptr; };
+  const int ff_list_zs[3] = {umma_zband_zs(64), ana ? umma_tile_zt(n.up.kb[0], 64, UEPI_VRN) : 0, ana ? umma_tile_zt(n.up.kb[1], 64, UEPI_VRN) : 0};
   for (int b0 = 0; b0 < B; b0 += SB) {
     const int nb = std::min(SB, B - b0);
     int cur = BUF_A, nxt = BUF_B;
     if (ff) {
       prof_begin(ctx, "ff_classify", 0, (double)nb * 64 * 64 * 64);
-      CK(launch_ff_classify((const uint8_t*)cubes + (size_t)b0 * 64 * 64 * 64, nb, ctx->ff_rows, ctx->ff_masks, ctx->stream, &ctx->launches));
+      CK(launch_ff_classify((const uint8_t*)cubes + (size_t)b0 * 64 * 64 * 64, nb, ctx->ff_rows, ctx->ff_masks, ff_ls, ctx->stream, &ctx->launches));
+      // the units each kernel computes or restores, shared by its persistent CTAs (a static split over all units leaves some CTAs with
+      // most of the near tiles)
+      FfListJob jobs;
+      for (int i = 0; i < 3; ++i) {
+        jobs.l[2 * i] = {ff_cur(2 * i + 1), ff_old(2 * i + 1), ff_list(2 * i), ff_list_zs[0]};
+        if (i < 2) jobs.l[2 * i + 1] = {ff_cur(2 * i + 2), ff_old(2 * i + 2), ff_list(2 * i + 1), ff_list_zs[1 + i]};
+      }
+      CK(launch_ff_list(jobs, 5, nb, ctx->stream, &ctx->launches));
       prof_end(ctx);
     }
+    auto act = [&](int L) { PmTensor t; t.p = (__nv_bfloat16*)ctx->ff_act[L]; t.n = 64; t.c = ff_ch[L]; t.B = nb; return t; };
     auto vrn_stage = [&](int stage, int C, int nn, bool s2d_last = false) -> int {
       for (int i = 0; i < 3; ++i) {
         const int idx = stage * 3 + i;
         int rr = umma("vrn_a", up.ka[idx], pm(cur, nn, C, nb), UEPI_PM, EPI_RELU, pm(BUF_T1, nn, C / 2, nb), none, nullptr, 0);
         if (rr) return rr;
         const bool s2d = s2d_last && i == 2;          // the block feeding a stride-2 conv writes its output space-to-depth
-        const bool ff_here = ff && stage == 0 && nn == 64;
         rr = umma("vrn_b", up.kb[idx], pm(BUF_T1, nn, C / 2, nb), UEPI_VRN, 0, s2d ? pm(nxt, nn / 2, 8 * C, nb) : pm(nxt, nn, C, nb),
-                  pm(cur, nn, C, nb), nullptr, 0, s2d, ff_here ? ctx->ff_masks + (size_t)i * nb * 128 : nullptr, ff_here ? ctx->ff_e[i] : nullptr);
+                  pm(cur, nn, C, nb), nullptr, 0, s2d);
         if (rr) return rr;
-        if (ana && ctx->ff_building && stage == 0 && nn == 64)      // the empty cube's block output (one cube: nb == 1)
-          CK(cudaMemcpyAsync(ctx->ff_e[i], ctx->bufs[nxt], ff_cube_bytes, cudaMemcpyDeviceToDevice, ctx->stream));
         std::swap(cur, nxt);
       }
       return PCGC_OK;
@@ -588,12 +623,27 @@ int run_vox_umma(pcgc_ctx* ctx, int kind, const float* in_ext, const void* cubes
         LayerW& lin = n.w[n.find("conv_in")];
         prof_begin(ctx, "conv_in_pm c1->16 n64", 2.0 * nb * in_elems * 27 * 16, 0);
         CK(launch_conv_in_pm((const char*)cubes + (size_t)b0 * in_elems * esz, cubes_dtype, lin.hk.data(), lin.hb.empty() ? nullptr : lin.hb.data(),
-                             ctx->bufs[cur], nb, ctx->stream, &ctx->launches));
+                             ctx->ff_act[0], nb, ff_cur(0), ff_old(0), ctx->stream, &ctx->launches));
         prof_end(ctx);
       }
-      if ((r = vrn_stage(0, 16, 64, true))) return r;
-      if ((r = umma("down_1", up.down[0], pm(cur, 32, 128, nb), UEPI_PM, EPI_RELU, pm(nxt, 32, 32, nb), none, nullptr, 0))) return r;
-      std::swap(cur, nxt);
+      // the three VRN-16 blocks: X_{2i} -> K_a -> T = layer 2i+1 -> K_b (+ residual X_{2i}) -> layer 2i+2; X3 (space-to-depth for down_1)
+      // goes to the shared buffer, every far tile of it copied
+      for (int i = 0; i < 3; ++i) {
+        const int L = 2 * i + 1;
+        if ((r = umma("vrn_a", up.ka[i], act(L - 1), UEPI_PM, EPI_RELU, act(L), none, nullptr, 0, 0, nullptr, nullptr, nullptr, ff_list(2 * i),
+                      ff_list_zs[0])))
+          return r;
+        const PmTensor out = i < 2 ? act(L + 1) : pm(BUF_B, 32, 128, nb);
+        if ((r = umma("vrn_b", up.kb[i], act(L), UEPI_VRN, 0, out, act(L - 1), nullptr, 0, i == 2, ff_cur(L + 1), ff_old(L + 1), ctx->ff_e[i],
+                      i < 2 ? ff_list(2 * i + 1) : nullptr, i < 2 ? ff_list_zs[1 + i] : 0)))
+          return r;
+        if (ctx->ff_building)                          // the empty cube's block output (one cube: nb == 1)
+          CK(cudaMemcpyAsync(ctx->ff_e[i], out.p, ff_cube_bytes, cudaMemcpyDeviceToDevice, ctx->stream));
+      }
+      if (ff) {                                        // the masks of these cubes describe their slots now; later slots keep theirs
+        CK(cudaMemcpy2DAsync(ctx->ff_prev, ff_ls, ctx->ff_masks, ff_ls, (size_t)nb * 128, 6, cudaMemcpyDeviceToDevice, ctx->stream));
+      }
+      if ((r = umma("down_1", up.down[0], pm(BUF_B, 32, 128, nb), UEPI_PM, EPI_RELU, pm(BUF_A, 32, 32, nb), none, nullptr, 0))) return r;
       if ((r = vrn_stage(1, 32, 32, true))) return r;
       if ((r = umma("down_2", up.down[1], pm(cur, 16, 256, nb), UEPI_PM, EPI_RELU, pm(nxt, 16, 64, nb), none, nullptr, 0))) return r;
       std::swap(cur, nxt);
@@ -1012,6 +1062,9 @@ void pcgc_destroy(pcgc_ctx* ctx) {
   for (auto e : ctx->ff_e) if (e) cudaFree(e);
   if (ctx->ff_rows) cudaFree(ctx->ff_rows);
   if (ctx->ff_masks) cudaFree(ctx->ff_masks);
+  if (ctx->ff_prev) cudaFree(ctx->ff_prev);
+  if (ctx->ff_lists) cudaFree(ctx->ff_lists);
+  for (auto a : ctx->ff_act) if (a) cudaFree(a);
   if (ctx->scratch) cudaFree(ctx->scratch);
   if (ctx->pmf_dev) cudaFree(ctx->pmf_dev);
   if (ctx->err_flag) cudaFree(ctx->err_flag);
@@ -1121,7 +1174,7 @@ int pcgc_load_conv(pcgc_ctx* ctx, int net, const char* layer, const float* kerne
   lw.hk.assign(kernel, kernel + (size_t)k * k * k * s.cin * s.cout);
   if (bias) lw.hb.assign(bias, bias + s.cout); else lw.hb.clear();
   n.up.ready = false;
-  if (net == PCGC_NET_VOX_ANALYSIS) ctx->ff_ready = false;        // the empty cube's activations belong to the old weights
+  if (net == PCGC_NET_VOX_ANALYSIS) ctx->ff_ready = ctx->ff_known = false;   // the empty cube's activations and the slots belong to the old weights
   if (n.up.conv_in_w) { cudaFree(n.up.conv_in_w); n.up.conv_in_w = nullptr; }
   for (int c = 0; c < lw.n_classes; ++c) if (lw.cls[c].w) { cudaFree((void*)lw.cls[c].w); lw.cls[c].w = nullptr; }
   if (lw.bias) { cudaFree(lw.bias); lw.bias = nullptr; }

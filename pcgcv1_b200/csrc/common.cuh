@@ -71,8 +71,10 @@ struct ConvCall {
 };
 
 cudaError_t launch_conv_ffma(const ConvCall& c, cudaStream_t s, int64_t* launches);
+// ff_mask / ff_prev (uint8 cubes only, or both nullptr): far-field masks of radius 1 (umma_conv.cuh launch_ff_classify) of these cubes
+// and of the cubes the output slots held before; voxels clear in both keep the empty cube's values already in out_pm and are not stored.
 cudaError_t launch_conv_in_pm(const void* cubes, int dtype, const float* w_host, const float* bias_host, void* out_pm, int B,
-                              cudaStream_t s, int64_t* launches);
+                              const uint8_t* ff_mask, const uint8_t* ff_prev, cudaStream_t s, int64_t* launches);
 cudaError_t launch_u8_to_f32(const void* in, int dtype, float* out, int64_t n, cudaStream_t s, int64_t* launches);
 
 // entropy.cu

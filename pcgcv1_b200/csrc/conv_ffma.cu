@@ -295,11 +295,14 @@ cudaError_t launch_conv_ffma(const ConvCall& c, cudaStream_t s, int64_t* launche
 // The 27x16 weights + bias travel as a by-value kernel parameter: they sit in the constant bank and every FFMA takes its
 // weight as a constant operand (no shared-memory weight loads; the first version was LDS.128-bound at 9 TFLOP/s).
 // r02 last session: all-zero taps are skipped per warp (see the loop).
+// Far-field voxels (ff_mask): a voxel with no occupied voxel within radius 1 is the empty cube's; it is stored only where the slot's
+// previous cube left it different (ff_prev), and a CTA none of whose voxels is stored returns at once.
 struct ConvInParams { float w[27 * 16]; float b[16]; };
 
 template <typename T>
 __global__ void __launch_bounds__(256) conv_in_pm_kernel(const T* __restrict__ in, const __grid_constant__ ConvInParams prm,
-                                                         __nv_bfloat16* __restrict__ out) {
+                                                         __nv_bfloat16* __restrict__ out, const uint8_t* __restrict__ ff_mask,
+                                                         const uint8_t* __restrict__ ff_prev) {
   constexpr int N = 64, TZ = 4, TY = 8;
   __shared__ float s_in[TZ + 2][TY + 2][N + 2];
   const int tid = threadIdx.x;
@@ -307,6 +310,14 @@ __global__ void __launch_bounds__(256) conv_in_pm_kernel(const T* __restrict__ i
   const int by = bid % (N / TY); bid /= (N / TY);
   const int bz = bid % (N / TZ); bid /= (N / TZ);
   const int b = bid;
+  // mask byte of (b, z, 32-line y tile): bit = 8-voxel x tile; the CTA's 8 lines lie in one y tile
+  const size_t m0 = ((size_t)b * N + bz * TZ) * 2 + (by * TY) / 32;
+  if (ff_mask) {
+    uint32_t any = 0;
+#pragma unroll
+    for (int zi = 0; zi < TZ; ++zi) any |= ff_mask[m0 + 2 * zi] | ff_prev[m0 + 2 * zi];
+    if (!any) return;                                              // CTA-uniform, before the barrier
+  }
   const T* ib = in + (size_t)b * N * N * N;
   for (int i = tid; i < (TZ + 2) * (TY + 2) * (N + 2); i += 256) {
     const int x = i % (N + 2), y = (i / (N + 2)) % (TY + 2), z = i / ((N + 2) * (TY + 2));
@@ -319,6 +330,8 @@ __global__ void __launch_bounds__(256) conv_in_pm_kernel(const T* __restrict__ i
   const int x = tid & 63, z = tid >> 6;
   const size_t pe = (size_t)N * N * N * 8;
   __nv_bfloat16* ob = out + (size_t)b * 4 * pe;
+  const bool store = !ff_mask || (((ff_mask[m0 + 2 * z] | ff_prev[m0 + 2 * z]) >> (x >> 3)) & 1u);
+  if (!__any_sync(0xFFFFFFFFu, store)) return;                    // warp-uniform; no barrier follows
 #pragma unroll 1
   for (int yy = 0; yy < 4; ++yy) {
     float a0[16], a1[16];
@@ -339,6 +352,7 @@ __global__ void __launch_bounds__(256) conv_in_pm_kernel(const T* __restrict__ i
     }
 #pragma unroll
     for (int c = 0; c < 16; ++c) { a0[c] = fmaxf(a0[c], 0.f); a1[c] = fmaxf(a1[c], 0.f); }
+    if (!store) continue;
     const int gz = bz * TZ + z, gy0 = by * TY + yy, gy1 = gy0 + 4;
     __nv_bfloat16* o0 = ob + (((size_t)gz * N + gy0) * N + x) * 8;
     __nv_bfloat16* o1 = ob + (((size_t)gz * N + gy1) * N + x) * 8;
@@ -349,16 +363,17 @@ __global__ void __launch_bounds__(256) conv_in_pm_kernel(const T* __restrict__ i
 
 // w: HOST float [27][16] tap-major (the Keras [3,3,3,1,16] kernel as is), bias HOST [16] or null.
 cudaError_t launch_conv_in_pm(const void* cubes, int dtype, const float* w_host, const float* bias_host, void* out_pm, int B,
-                              cudaStream_t s, int64_t* launches) {
+                              const uint8_t* ff_mask, const uint8_t* ff_prev, cudaStream_t s, int64_t* launches) {
+  if ((ff_mask != nullptr) != (ff_prev != nullptr) || (ff_mask && dtype != PCGC_DTYPE_U8)) return cudaErrorInvalidValue;
   ConvInParams prm;
   for (int i = 0; i < 27 * 16; ++i) prm.w[i] = w_host[i];
   for (int i = 0; i < 16; ++i) prm.b[i] = bias_host ? bias_host[i] : 0.f;
   const int grid = (64 / 8) * (64 / 4) * B;
   if (launches) ++*launches;
   switch (dtype) {
-    case PCGC_DTYPE_U8: PCGC_CARVEOUT_ONCE(conv_in_pm_kernel<uint8_t>); conv_in_pm_kernel<uint8_t><<<grid, 256, 0, s>>>((const uint8_t*)cubes, prm, (__nv_bfloat16*)out_pm); break;
-    case PCGC_DTYPE_F32: conv_in_pm_kernel<float><<<grid, 256, 0, s>>>((const float*)cubes, prm, (__nv_bfloat16*)out_pm); break;
-    case PCGC_DTYPE_F64: conv_in_pm_kernel<double><<<grid, 256, 0, s>>>((const double*)cubes, prm, (__nv_bfloat16*)out_pm); break;
+    case PCGC_DTYPE_U8: PCGC_CARVEOUT_ONCE(conv_in_pm_kernel<uint8_t>); conv_in_pm_kernel<uint8_t><<<grid, 256, 0, s>>>((const uint8_t*)cubes, prm, (__nv_bfloat16*)out_pm, ff_mask, ff_prev); break;
+    case PCGC_DTYPE_F32: conv_in_pm_kernel<float><<<grid, 256, 0, s>>>((const float*)cubes, prm, (__nv_bfloat16*)out_pm, nullptr, nullptr); break;
+    case PCGC_DTYPE_F64: conv_in_pm_kernel<double><<<grid, 256, 0, s>>>((const double*)cubes, prm, (__nv_bfloat16*)out_pm, nullptr, nullptr); break;
     default: return cudaErrorInvalidValue;
   }
   return cudaGetLastError();

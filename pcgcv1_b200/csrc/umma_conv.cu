@@ -77,10 +77,16 @@ struct UmmaArgs {
   int out_s2d;               // UEPI_VRN: write the output space-to-depth (grid n/2, 8*C channels) for a following stride-2 conv
   int up_ncls, up_cls0, up_cout;   // UEPI_UP: classes in this launch, first class, channels per class
   int dbg;                   // PCGC_UMMA_DBG bit mask (timing experiments only): 1 skip MMAs, 2 skip the A TMA, 4 skip epilogue
-  // far-field tiles (tile kernel, UEPI_VRN on the 64^3 grid): ff_mask[(b*n + z)*ty_n + by] bit bx = 1 when some occupied voxel lies inside the
-  // receptive field of that (z, y tile, x tile); a tile whose zt slices are all clear is COPIED from ff_src, the same layer's output for
-  // the all-zero cube (one cube, same layout as out_pm) -- bit-identical to computing it.  nullptr: every tile is computed.
-  const uint8_t* ff_mask; const __nv_bfloat16* ff_src;
+  // far-field tiles of the analysis 64^3 stage: ff_mask[(b*n + z)*ty_n + by] bit bx = 1 when some occupied voxel lies inside the receptive
+  // field of that (z, y tile, x tile) of the output layer; ff_prev is the same mask of the cube the output slot held before (the slot
+  // holds the empty cube's values wherever that bit is clear), or nullptr when the slot holds nothing known.
+  //   tile kernel (UEPI_VRN): a tile whose zt slices are all clear in ff_mask is not computed.  It is COPIED from ff_src, the same
+  //     layer's output for the all-zero cube (one cube, same layout as out_pm), unless it is clear in ff_prev too: then nothing is written.
+  //   z-banded kernel (UEPI_PM): the segments (ZS slices) clear in both masks are left out of ff_list; every listed segment is computed whole.
+  // ff_list = {count, unit indices in the kernel's tile / segment numbering} (launch_ff_list): the tiles or segments the persistent CTAs
+  // share; nullptr: all of them.  Bit-identical to computing every tile.  ff_mask nullptr: every tile is computed.
+  const uint8_t* ff_mask; const uint8_t* ff_prev; const __nv_bfloat16* ff_src;
+  const int* ff_list;
   // z-streaming kernel (conv_umma_stream_kernel)
   int ring, zs, nacc;        // input-slice ring slots, output slices per segment, accumulator slots
   int slot_bytes;            // bytes of one ring slot = planes * slice_plane
@@ -332,7 +338,8 @@ __global__ void __launch_bounds__(UMMA_THREADS, (NP <= 16 ? 3 : (NP <= 32 ? 2 : 
   constexpr int NPJ = NP / WT;                       // accumulator columns per output line j
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int tx_n = a.n / TILE_X, ty_n = a.n / (TILE_Y * WT), tz_n = a.n / a.zt;
-  const int total_tiles = tx_n * ty_n * tz_n * a.batch;
+  constexpr bool FFL = EPI == UEPI_VRN && WT == 2;             // the only form launched with a far-field list (K_b16)
+  const int total_tiles = (FFL && a.ff_list) ? a.ff_list[0] : tx_n * ty_n * tz_n * a.batch;   // far-field tiles: the listed ones only
   const uint32_t set_cols = (uint32_t)(a.zt * 2 * NP);
 
   for (int i = tid; i < NP; i += UMMA_THREADS) s_bias[i] = a.bias ? a.bias[i] : 0.f;
@@ -369,7 +376,7 @@ __global__ void __launch_bounds__(UMMA_THREADS, (NP <= 16 ? 3 : (NP <= 32 ? 2 : 
       uint32_t n_full = 0, n_mma = 0;                  // completed phases of bar_full / bar_mma
       int it = 0;
       for (int tile = blockIdx.x; tile < total_tiles && alive; tile += gridDim.x) {
-        int r = tile;
+        int r = (FFL && a.ff_list) ? a.ff_list[1 + tile] : tile;
         const int bx = r % tx_n; r /= tx_n;
         const int by = r % ty_n; r /= ty_n;
         const int bz = r % tz_n; r /= tz_n;
@@ -409,7 +416,7 @@ __global__ void __launch_bounds__(UMMA_THREADS, (NP <= 16 ? 3 : (NP <= 32 ? 2 : 
     const size_t plane_elems = (size_t)a.n * a.n * a.n * 8;
     int it = 0;
     for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-      int r = tile;
+      int r = (FFL && a.ff_list) ? a.ff_list[1 + tile] : tile;
       const int bx = r % tx_n; r /= tx_n;
       const int by = r % ty_n; r /= ty_n;
       const int bz = r % tz_n; r /= tz_n;
@@ -418,8 +425,10 @@ __global__ void __launch_bounds__(UMMA_THREADS, (NP <= 16 ? 3 : (NP <= 32 ? 2 : 
       const int vx = x0 + (row & 7), vyb = y0 + WT * (row >> 3);
       if constexpr (EPI == UEPI_VRN) {
         if (a.ff_mask && ff_tile_clear(a.ff_mask, a.n, a.zt, b, by, bx, z0, ty_n)) {
-          // far-field tile: no MMA, no barrier -- every voxel is the empty cube's at the same position
-          for (int zi = (warp >> 2); zi < a.zt; zi += 2) ff_copy_voxels<NPJ, WT>(a, b, z0 + zi, vyb, vx, plane_elems);
+          // far-field tile: no MMA, no barrier -- every voxel is the empty cube's at the same position, which the slot already holds
+          // where the tile was far for its previous cube as well
+          if (!a.ff_prev || !ff_tile_clear(a.ff_prev, a.n, a.zt, b, by, bx, z0, ty_n))
+            for (int zi = (warp >> 2); zi < a.zt; zi += 2) ff_copy_voxels<NPJ, WT>(a, b, z0 + zi, vyb, vx, plane_elems);
           continue;
         }
       }
@@ -750,7 +759,11 @@ __global__ void __launch_bounds__(32 * (4 * EG + 1 + NI), 1) conv_umma_zband_ker
   const int RMASK = a.ring - 1, RSH = a.ring == 8 ? 3 : 2;
   const int tx_n = a.n / TILE_X, ty_n = a.n / (TILE_Y * WT), tz_n = a.n / ZS;
   const int total_segs = tx_n * ty_n * tz_n * a.batch;
-  const int n_my = ((int)blockIdx.x < total_segs) ? (total_segs - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
+  // far-field segments (UmmaArgs::ff_list): the CTAs share the list of the segments to compute, so that the work is balanced however the
+  // occupied voxels lie; loads, outputs and barrier phases count listed segments only
+  const int n_units = a.ff_list ? a.ff_list[0] : total_segs;
+  const int n_my = ((int)blockIdx.x < n_units) ? (n_units - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
+  auto seg_of = [&](int sk) -> int { const int u = (int)blockIdx.x + sk * (int)gridDim.x; return a.ff_list ? a.ff_list[1 + u] : u; };
   const int total_outs = n_my * ZS, total_loads = n_my * LPS;
 
   for (int i = tid; i < NP; i += THREADS) s_bias[i] = a.bias ? a.bias[i] : 0.f;
@@ -782,7 +795,7 @@ __global__ void __launch_bounds__(32 * (4 * EG + 1 + NI), 1) conv_umma_zband_ker
       int l = 0;
       bool alive = true;
       for (int sk = 0; sk < n_my && alive; ++sk) {
-        int r = (int)blockIdx.x + sk * (int)gridDim.x;
+        int r = seg_of(sk);
         const int bx = r % tx_n; r /= tx_n;
         const int by = r % ty_n; r /= ty_n;
         const int bz = r % tz_n; r /= tz_n;
@@ -862,7 +875,7 @@ __global__ void __launch_bounds__(32 * (4 * EG + 1 + NI), 1) conv_umma_zband_ker
     while (o >= ZS) { o -= ZS; ++sk; }
     for (int O = (warp >> 2); O < ((a.dbg & 4) ? 0 : total_outs); O += EG) {
       if (sk != cur) {
-        int r = (int)blockIdx.x + sk * (int)gridDim.x;
+        int r = seg_of(sk);
         bx = r % tx_n; r /= tx_n;
         by = r % ty_n; r /= ty_n;
         bz = r % tz_n; r /= tz_n;
@@ -1182,7 +1195,7 @@ cudaError_t launch_conv_umma_pm(const UmmaCall& c, const UmmaWeights& w, cudaStr
   a.w23 = w.w23; a.b23 = w.b23; a.c4 = w.c4; a.c2 = w.c2;
   a.up_ncls = w.up_ncls; a.up_cls0 = w.up_cls0; a.up_cout = w.up_cout;
   a.origin = w.origin; a.out_s2d = c.out_s2d;
-  a.ff_mask = nullptr; a.ff_src = nullptr;               // set below, on the tile-kernel path only
+  a.ff_mask = nullptr; a.ff_prev = nullptr; a.ff_src = nullptr; a.ff_list = nullptr;   // set below, on the paths that read them
   for (int i = 0; i < 16; ++i) a.tap_mask[i] = w.tap_mask[i];
   a.err = c.err;
   { static const int dbg = getenv("PCGC_UMMA_DBG") ? atoi(getenv("PCGC_UMMA_DBG")) : 0; a.dbg = dbg; }
@@ -1205,11 +1218,12 @@ cudaError_t launch_conv_umma_pm(const UmmaCall& c, const UmmaWeights& w, cudaStr
     const size_t budget = (size_t)220 * 1024;
     const int z_ring = (size_t)8 * z_slot + fixed <= budget ? 8 : ((size_t)4 * z_slot + fixed <= budget ? 4 : 0);
     if (z_ring) {
-      a.zs = n >= 64 ? 16 : 8;                                 // enough segments per launch to balance 148 persistent CTAs
+      a.zs = umma_zband_zs(n);                                 // enough segments per launch to balance 148 persistent CTAs
       a.slice_plane = z_slice_plane; a.slot_bytes = z_slot; a.ring = z_ring;
       a.b_bytes = w.zb_bytes;
       a.wpacked = (const __nv_bfloat16*)w.packed_zb;
       a.nacc = ZB_SLOTS; a.tmem_cols = 512; a.batch = c.in.B;
+      if (c.ff_list && c.ff_list_zs == a.zs && c.epi == UEPI_PM && w.wt == 2 && n == 64) a.ff_list = c.ff_list;   // K_a16
       CUtensorMap tmz;
       cudaError_t ez = make_tmap(c.in, brick_ey(w.wt), 1, a.ppc * w.kchunks, &tmz);
       if (ez != cudaSuccess) return ez;
@@ -1291,7 +1305,10 @@ cudaError_t launch_conv_umma_pm(const UmmaCall& c, const UmmaWeights& w, cudaStr
   static const int persist = getenv("PCGC_UMMA_PERSIST") ? atoi(getenv("PCGC_UMMA_PERSIST")) : 1;  // 0: one tile per CTA
   const int grid = persist ? std::min(tiles, sms * per_sm) : tiles;
   if (launches) ++*launches;
-  if (c.ff_mask && c.ff_src && c.epi == UEPI_VRN && w.wt == 2 && n == 64) { a.ff_mask = c.ff_mask; a.ff_src = c.ff_src; }
+  if (c.ff_mask && c.ff_src && c.epi == UEPI_VRN && w.wt == 2 && n == 64) {
+    a.ff_mask = c.ff_mask; a.ff_prev = c.ff_prev; a.ff_src = c.ff_src;
+    if (c.ff_list && c.ff_list_zs == a.zt) a.ff_list = c.ff_list;
+  }
   if (w.wt > 1) return launch_banded(tm, a, w.np, c.epi, a.cin8 != 0, w.wt, grid, smem, s);
   if (c.epi == UEPI_UP) {
     if (w.ntaps != 8 || w.np != 128) return cudaErrorNotSupported;
@@ -1318,7 +1335,7 @@ cudaError_t launch_conv_umma_pm(const UmmaCall& c, const UmmaWeights& w, cudaStr
 }
 
 // ---------------------------------------------------------------------------------------------- far-field classification
-// Kernel 1: one thread per row (b, z, y): the 64 occupancy bytes -> a 64-bit mask, dilated along x by r = 3 / 5 / 7 (shifts drop what
+// Kernel 1: one thread per row (b, z, y): the 64 occupancy bytes -> a 64-bit mask, dilated along x by r = 1 .. FF_LAYERS (shifts drop what
 // leaves the cube, like the zero padding) and collapsed to one bit per 8-voxel x tile.
 __global__ void __launch_bounds__(256) ff_row_mask_kernel(const uint8_t* __restrict__ cubes, int rows, uint8_t* __restrict__ row_mask) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1336,11 +1353,9 @@ __global__ void __launch_bounds__(256) ff_row_mask_kernel(const uint8_t* __restr
         if ((w[k] >> (8 * bb)) & 0xFFu) m |= 1ull << (q * 16 + k * 4 + bb);
   }
   uint64_t d = m;
-  int done = 0;
 #pragma unroll
-  for (int k = 0; k < 3; ++k) {
-    const int r = 3 + 2 * k;
-    for (; done < r; ++done) d |= (d << 1) | (d >> 1);             // one more voxel of dilation per step
+  for (int k = 0; k < FF_LAYERS; ++k) {
+    d |= (d << 1) | (d >> 1);                                      // one more voxel of dilation per layer
     uint32_t t = 0;
 #pragma unroll
     for (int bx = 0; bx < 8; ++bx) t |= ((d >> (8 * bx)) & 0xFFull) ? (1u << bx) : 0u;
@@ -1348,30 +1363,82 @@ __global__ void __launch_bounds__(256) ff_row_mask_kernel(const uint8_t* __restr
   }
 }
 // Kernel 2: one thread per (k, b, z, by): OR of the row masks over z +- r and the tile's 32 lines +- r.
-__global__ void __launch_bounds__(128) ff_tile_mask_kernel(const uint8_t* __restrict__ row_mask, int nb, uint8_t* __restrict__ ff_mask) {
+__global__ void __launch_bounds__(128) ff_tile_mask_kernel(const uint8_t* __restrict__ row_mask, int nb, size_t layer_stride, uint8_t* __restrict__ ff_mask) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   const int per = nb * 128;
-  if (i >= 3 * per) return;
+  if (i >= FF_LAYERS * per) return;
   const int k = i / per, j = i - k * per;
   const int by = j & 1, z = (j >> 1) & 63, b = j >> 7;
-  const int r = 3 + 2 * k;
+  const int r = k + 1;
   const uint8_t* rm = row_mask + (size_t)k * nb * 4096 + (size_t)b * 4096;
   const int z0 = max(z - r, 0), z1 = min(z + r, 63), y0 = max(32 * by - r, 0), y1 = min(32 * by + 31 + r, 63);
   uint32_t t = 0;
   for (int zz = z0; zz <= z1; ++zz)
     for (int yy = y0; yy <= y1; ++yy) t |= rm[zz * 64 + yy];
-  ff_mask[i] = (uint8_t)t;
+  ff_mask[(size_t)k * layer_stride + j] = (uint8_t)t;
 }
 
-cudaError_t launch_ff_classify(const uint8_t* cubes, int nb, uint8_t* row_mask, uint8_t* ff_mask, cudaStream_t s, int64_t* launches) {
+cudaError_t launch_ff_classify(const uint8_t* cubes, int nb, uint8_t* row_mask, uint8_t* ff_mask, size_t layer_stride, cudaStream_t s, int64_t* launches) {
   if (nb <= 0) return cudaSuccess;
   PCGC_CARVEOUT_ONCE(ff_row_mask_kernel); PCGC_CARVEOUT_ONCE(ff_tile_mask_kernel);
   const int rows = nb * 4096;
   ff_row_mask_kernel<<<(rows + 255) / 256, 256, 0, s>>>(cubes, rows, row_mask);
-  ff_tile_mask_kernel<<<(3 * nb * 128 + 127) / 128, 128, 0, s>>>(row_mask, nb, ff_mask);
+  ff_tile_mask_kernel<<<(FF_LAYERS * nb * 128 + 127) / 128, 128, 0, s>>>(row_mask, nb, layer_stride, ff_mask);
   if (launches) *launches += 2;
   return cudaGetLastError();
 }
+
+// Kernel 3 (launch_ff_list): one CTA per list.  Unit u = ((b*(64/zs) + bz)*2 + by)*8 + bx (zs slices of an 8 x 32-voxel tile, the kernels'
+// tile / segment numbering) is listed when any of its slices is set in mask | prev; ordered compaction, list[0] = count.
+__global__ void __launch_bounds__(1024) ff_list_kernel(FfListJob jobs, int nb) {
+  const FfListJob::One& j = jobs.l[blockIdx.x];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tz_n = 64 / j.zs, units = nb * tz_n * 16;
+  __shared__ int s_warp[32];
+  __shared__ int s_base;
+  if (tid == 0) s_base = 0;
+  __syncthreads();
+  for (int c0 = 0; c0 < units; c0 += 1024) {
+    const int u = c0 + tid;
+    bool act = false;
+    if (u < units) {
+      const int bx = u & 7, by = (u >> 3) & 1, bz = (u >> 4) % tz_n, b = (u >> 4) / tz_n;
+      const size_t o = ((size_t)b * 64 + bz * j.zs) * 2 + by;
+      uint32_t t = 0;
+      for (int zi = 0; zi < j.zs; ++zi) t |= j.mask[o + 2 * zi] | j.prev[o + 2 * zi];
+      act = (t >> bx) & 1u;
+    }
+    const uint32_t bal = __ballot_sync(0xFFFFFFFFu, act);
+    if (lane == 0) s_warp[warp] = __popc(bal);
+    __syncthreads();
+    if (warp == 0) {
+      const int v = s_warp[lane];
+      int inc = v;
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) { const int t2 = __shfl_up_sync(0xFFFFFFFFu, inc, d); if (lane >= d) inc += t2; }
+      s_warp[lane] = inc - v;                                      // exclusive prefix of the warp counts
+    }
+    __syncthreads();
+    if (act) j.list[1 + s_base + s_warp[warp] + __popc(bal & ((1u << lane) - 1u))] = u;
+    __syncthreads();
+    if (tid == 1023) s_base += s_warp[31] + __popc(bal);           // the last warp's prefix + its count
+    __syncthreads();
+  }
+  if (tid == 0) j.list[0] = s_base;
+}
+
+cudaError_t launch_ff_list(const FfListJob& jobs, int n_jobs, int nb, cudaStream_t s, int64_t* launches) {
+  if (nb <= 0 || n_jobs <= 0) return cudaSuccess;
+  if (n_jobs > FfListJob::MAX) return cudaErrorInvalidValue;
+  for (int i = 0; i < n_jobs; ++i) if (jobs.l[i].zs < 1 || 64 % jobs.l[i].zs) return cudaErrorInvalidValue;
+  PCGC_CARVEOUT_ONCE(ff_list_kernel);
+  ff_list_kernel<<<n_jobs, 1024, 0, s>>>(jobs, nb);
+  if (launches) ++*launches;
+  return cudaGetLastError();
+}
+
+int umma_tile_zt(const UmmaWeights& w, int n, int epi) { return pick_zt(n, w.np, w.cin, epi, w.wt, w.n_mma, w.kchunks); }
+int umma_zband_zs(int n) { return n >= 64 ? 16 : 8; }
 
 // ---------------------------------------------------------------------------------------------- format converters
 __global__ void f32_to_pm_kernel(const float* __restrict__ in, int in_cs, int in_co, __nv_bfloat16* __restrict__ out,

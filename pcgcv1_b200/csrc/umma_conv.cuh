@@ -61,9 +61,14 @@ struct UmmaCall {
   PmTensor res;                // UEPI_VRN: the block input x
   int out_s2d = 0;             // UEPI_VRN: write `out` space-to-depth (out = the n/2-grid, 8*C-channel tensor)
   int* err = nullptr;          // device int, set on device-side timeouts
-  // far-field tiles (UEPI_VRN on the tile kernel, 64^3 grid, y-band 2): mask from launch_ff_classify for this layer's radius + the layer's
-  // output for the all-zero cube; see UmmaArgs::ff_mask.  Ignored (every tile computed) by the other kernel forms.
-  const uint8_t* ff_mask = nullptr; const __nv_bfloat16* ff_src = nullptr;
+  // far-field tiles of the analysis 64^3 stage (y-band 2): masks from launch_ff_classify for the output layer's radius, of the current
+  // cubes (ff_mask) and of the cubes the output slots held before (ff_prev); the layer's output for the all-zero cube (ff_src).  Read by
+  // the tile kernel's UEPI_VRN form (K_b16); the z-banded kernel's UEPI_PM form (K_a16) reads only ff_list.  See UmmaArgs::ff_mask.
+  // Ignored (every tile computed) by the other kernel forms.
+  const uint8_t* ff_mask = nullptr; const uint8_t* ff_prev = nullptr; const __nv_bfloat16* ff_src = nullptr;
+  // the units to compute or restore (launch_ff_list, built with zs = ff_list_zs slices per unit); used only where ff_list_zs is the
+  // kernel's own z extent (umma_tile_zt / umma_zband_zs), otherwise every unit is visited
+  const int* ff_list = nullptr; int ff_list_zs = 0;
   bool pin_tile = false;       // always the tile kernel, whatever PCGC_UMMA_STREAM / PCGC_UMMA_ZBAND / PCGC_KB_ZBAND say: the hyper
                                // decoder's loc / scale must have the same bits in the encoding and the decoding process
 };
@@ -73,10 +78,22 @@ cudaError_t launch_conv_umma_pm(const UmmaCall& c, const UmmaWeights& w, cudaStr
 int umma_stream_mode();
 // PCGC_UMMA_ZBAND (default 1, needs streaming): z-banded kernel for the NP = 16 layers (K_a16, K_a32, K_b16, deconv_out)
 int umma_zband_mode();
-// Far-field classification of a batch of uint8 occupancy cubes [nb][64][64][64] for the three VRN-16 blocks of the analysis transform
-// (receptive-field radii 3, 5, 7 voxels): ff_mask[k][(b*64 + z)*2 + by] bit bx = 1 when an occupied voxel lies within radius r_k of the
-// 8 (x) x 32 (y) voxels of tile (by, bx) in slice z.  row_mask: scratch [3][nb*4096] bytes; ff_mask: [3][nb*128] bytes.
-cudaError_t launch_ff_classify(const uint8_t* cubes, int nb, uint8_t* row_mask, uint8_t* ff_mask, cudaStream_t s, int64_t* launches);
+// Far-field classification of a batch of uint8 occupancy cubes [nb][64][64][64] for the seven layers of the analysis 64^3 stage (conv_in
+// output, then K_a and K_b of the three VRN-16 blocks: receptive-field radii 1 .. 7 voxels): ff_mask[k * layer_stride + (b*64 + z)*2 + by]
+// bit bx = 1 when an occupied voxel lies within radius k + 1 of the 8 (x) x 32 (y) voxels of tile (by, bx) in slice z.
+// row_mask: scratch [FF_LAYERS][nb*4096] bytes; layer_stride >= nb*128.
+constexpr int FF_LAYERS = 7;
+cudaError_t launch_ff_classify(const uint8_t* cubes, int nb, uint8_t* row_mask, uint8_t* ff_mask, size_t layer_stride, cudaStream_t s, int64_t* launches);
+// Work lists of the far-field kernels, one per job: the units (zs slices of an 8 x 32-voxel tile, numbered ((b*(64/zs) + bz)*2 + by)*8 + bx)
+// with a bit set in mask | prev, in increasing order: list = {count, units...}, room for nb*(64/zs)*16 + 1 ints.  One launch for all jobs.
+struct FfListJob {
+  static constexpr int MAX = 8;
+  struct One { const uint8_t* mask; const uint8_t* prev; int* list; int zs; } l[MAX];
+};
+cudaError_t launch_ff_list(const FfListJob& jobs, int n_jobs, int nb, cudaStream_t s, int64_t* launches);
+// z extent of a launch: slices per tile of the tile kernel, per segment of the z-banded kernel
+int umma_tile_zt(const UmmaWeights& w, int n, int epi);
+int umma_zband_zs(int n);
 // float32 NDHWC (channel stride/offset) <-> PM
 cudaError_t launch_f32_to_pm(const float* in, int in_cs, int in_co, const PmTensor& out, cudaStream_t s, int64_t* launches);
 cudaError_t launch_pm_to_f32(const PmTensor& in, float* out, int out_cs, int out_co, cudaStream_t s, int64_t* launches);
